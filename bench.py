@@ -485,6 +485,22 @@ def run_reference_vo(args, rank: int, world: int) -> None:
     print(json.dumps(line))
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, **arrays) -> None:
+    """Writes every array as <out_dir>/<name>.npy in float64.  The poses of one step take 96 bytes per frame, so the frames
+    the resident leg keeps in HBM (307 kB each) bound them far below DUMP_LIMIT_BYTES; the check makes sure of it."""
+    out = {k: np.asarray(v, np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes of outputs exceed {DUMP_LIMIT_BYTES}")
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    for k, a in out.items():
+        np.save(d / f"{k}.npy", a)
+
+
 def vo_gpu_leg(ctx, stacked, depths, threads, warm, device_ptr=None, window=8, engine="resident"):
     from ygz_slam_b200 import vo_native
     S, n = stacked.shape[:2]
@@ -564,6 +580,9 @@ def vo_line(args, rank, world, local_rank):
         barrier()
         remeasured = {"first_resident_ms": first_ms, "second_resident_ms": det_r["device_ms"], "e2e_ms": sec_e * 1e3,
                       "reason": "resident leg slower than 1.5x the e2e leg of the same frames"}
+    if args.dump_outputs and rank == 0:
+        # what the timed (resident) leg returned: the poses of its last step, and the per-stream counters of the run
+        dump_outputs(args.dump_outputs, poses=traj_r[:, n - F:], tracking_stats=[list(s.values()) for s in stats_r])
     # diagnostics (untimed legs of the same streams): one frame per stream in flight (the latency mode of the engine) and
     # the per-stage C-ABI path of round 1 (one blocking call per stage and lock-step frame)
     diag = {}
@@ -1051,7 +1070,16 @@ def main() -> None:
     ap.add_argument("--e2e-contexts", type=int, default=8,
                     help="extract_match: host threads (one ygzb context = one stream each) used by the e2e leg so that the H2D "
                          "copy of one batch overlaps the kernels of another")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="vo: after the timed steps, write what the timed leg computed as DIR/<name>.npy (float64): poses.npy = "
+                         "(streams, frames per step, 3, 4) camera poses T_cw of the last step, tracking_stats.npy = (streams, 12) "
+                         "per-stream counters (lost, keyframes, ba, candidates, projected, inliers, ba_obs, ba_pts, ba_kfs, "
+                         "ba_trials, ba_iters, ba_flops); rank 0's streams")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "vo"):
+        ap.error("--dump-outputs writes the outputs of the GPU path of the vo workload")
     if args.warmup < 3:
         args.warmup = 3
 

@@ -2,11 +2,12 @@
 
 The oracle (oracle/bow.cpp) follows the vendored DBoW3 source; here it is checked against an independent numpy descent
 written from the file format and the transform's text (Vocabulary.cpp:706-832, 1180-1225), on synthetic vocabularies in the
-same binary format and -- when the reference tree is present (this container, not the GPU box) -- on its own
-vocab/ORBvoc.bin.  The GPU tests compare the CUDA path with the oracle: word / node / match indices exact, values 1e-14.
+same binary format and on the part of the reference's own vocab/ORBvoc.bin that real descriptors descend through
+(tests/golden/orbvoc_subtree.npz).  The GPU tests compare the CUDA path with the oracle: word / node / match indices exact,
+values 1e-14.
 """
-import os
 import struct
+from pathlib import Path
 
 import numpy as np
 import pytest
@@ -14,7 +15,7 @@ import pytest
 from oracle.pyoracle import Oracle
 from ygz_slam_b200 import synth
 
-ORBVOC = "/root/reference/vocab/ORBvoc.bin"
+GOLD_VOC = Path(__file__).resolve().parent / "golden" / "orbvoc_subtree.npz"
 REC = np.dtype([("parent", "<i4"), ("desc", "u1", 32), ("w", "<f4"), ("leaf", "u1")])
 
 
@@ -130,22 +131,31 @@ def test_loader_rejects_malformed(ora):
         ora.vocab_load(bytes(bad))
 
 
-@pytest.mark.skipif(not os.path.exists(ORBVOC), reason="the reference's vocab/ORBvoc.bin is only present next to the reference tree")
 def test_oracle_on_reference_vocabulary(ora):
-    data = open(ORBVOC, "rb").read()
+    """The reference's vocab/ORBvoc.bin, reduced to the nodes that the descents of 150 real ORB descriptors (synthetic frame 2)
+    compare against (tools/make_orbvoc_fixture.py): the oracle and the numpy descent agree on the reduced tree, and mapped back
+    to the whole file's node and word ids they give what the whole file gave."""
+    g = np.load(GOLD_VOC)
+    assert tuple(g["info"]) == (10, 6, 0, 0, 1082075, 971816)                  # the whole file: k, L, L1_NORM, TF_IDF, nodes, words
+    data = g["vocab"].tobytes()
+    rec = parse(data)[0]
     v = ora.vocab_load(data)
     info = ora.vocab_info(v)
-    assert (info["k"], info["L"], info["scoring"], info["weighting"]) == (10, 6, 0, 0)   # L1_NORM, TF_IDF
-    assert info["nodes"] == 1082075 and info["words"] == 971816
+    assert (info["k"], info["L"], info["scoring"], info["weighting"]) == (10, 6, 0, 0)
+    assert info["nodes"] == len(rec) + 2 and info["words"] == int(rec["leaf"].sum()) + int(rec["leaf"][-1])
     # real ORB descriptors of a synthetic frame
-    g, _, _ = synth.stream_frame(2)
-    pyr = ora.build_pyramid(g, 3)
+    img, _, _ = synth.stream_frame(2)
+    pyr = ora.build_pyramid(img, 3)
     f = ora.detect(pyr, n_levels=3)
     desc = ora.describe(pyr, 640, 480, 3, f["px"], f["py"], f["level"])[1][:150]
-    word, node, weight, bw, bv = ora.bow_transform(v, desc, 4)
-    nw, nn, nwt, nbow = numpy_transform(data, desc, 4)
+    assert np.array_equal(desc, g["desc"])
+    word, node, weight, bw, bv = ora.bow_transform(v, desc, int(g["levelsup"]))
+    nw, nn, nwt, nbow = numpy_transform(data, desc, int(g["levelsup"]))
     assert np.array_equal(word, nw) and np.array_equal(node, nn) and np.array_equal(weight, nwt)
     assert list(bw) == sorted(nbow) and np.allclose(bv, [nbow[a] for a in sorted(nbow)], rtol=1e-15, atol=0)
+    assert np.array_equal(g["word_id"][word], g["word"]) and np.array_equal(np.where(node >= 0, g["node_id"][node], -1), g["node"])
+    assert np.array_equal(weight, g["weight"]) and (g["node"] >= 0).sum() > 100
+    assert np.array_equal(g["word_id"][bw], g["bow_words"]) and np.allclose(bv, g["bow_values"], rtol=1e-15, atol=0)
     assert abs(bv.sum() - 1.0) < 1e-12
     ora.vocab_free(v)
 
