@@ -7,30 +7,30 @@ import numpy as np
 import pytest
 
 ROOT = Path(__file__).resolve().parent.parent
-EXE = ROOT / "tests" / "_build" / "cpp_shim_test"
 
 
-def build_shim_test():
+@pytest.fixture(scope="module")
+def shim_exe(tmp_path_factory):
+    """The shim test binary, built in a temporary directory: the repository tree may be read-only."""
     from ygz_slam_b200 import capi
     capi.load_library()
-    EXE.parent.mkdir(exist_ok=True)
-    cmd = ["g++", "-std=c++17", "-O1", "-Wall", "-Werror", "-o", str(EXE), str(ROOT / "tests" / "cpp_shim_test.cpp"),
+    exe = tmp_path_factory.mktemp("cpp_shim") / "cpp_shim_test"
+    cmd = ["g++", "-std=c++17", "-O1", "-Wall", "-Werror", "-o", str(exe), str(ROOT / "tests" / "cpp_shim_test.cpp"),
            f"-L{ROOT / 'ygz_slam_b200'}", "-lygz_b200", f"-Wl,-rpath,{ROOT / 'ygz_slam_b200'}"]
     subprocess.run(cmd, check=True, capture_output=True, text=True)
+    return exe
 
 
-def test_shim_compiles_and_links_without_cuda_headers():
+def test_shim_compiles_and_links_without_cuda_headers(shim_exe):
     """Host C++ only needs include/ygz_b200.h + the shim header: no CUDA toolkit on the include path."""
-    build_shim_test()
-    assert EXE.exists()
-    r = subprocess.run([str(EXE)], capture_output=True)
+    assert shim_exe.exists()
+    r = subprocess.run([str(shim_exe)], capture_output=True)
     assert r.returncode == 2  # usage error, i.e. the binary starts and the shared library resolves
 
 
 @pytest.mark.gpu
-def test_shim_reproduces_oracle(oracle, tmp_path):
+def test_shim_reproduces_oracle(shim_exe, oracle, tmp_path):
     from ygz_slam_b200 import se3, synth
-    build_shim_test()
     g1, d1, T1 = synth.stream_frame(1)
     g2, _, T2 = synth.stream_frame(4)
     Trel = se3.mul(T2, se3.inv(T1))
@@ -45,7 +45,7 @@ def test_shim_reproduces_oracle(oracle, tmp_path):
     blob3 = tmp_path / "third.bin"
     with open(blob3, "wb") as f:
         f.write(g3.tobytes()); f.write(T31.astype(np.float64).tobytes())
-    r = subprocess.run([str(EXE), str(blob), str(voc_file), str(blob3)], capture_output=True, text=True, check=True)
+    r = subprocess.run([str(shim_exe), str(blob), str(voc_file), str(blob3)], capture_output=True, text=True, check=True)
     lines = r.stdout.strip().splitlines()
     f1 = oracle.detect(oracle.build_pyramid(g1, 3))
     f2 = oracle.detect(oracle.build_pyramid(g2, 3))

@@ -117,6 +117,36 @@ def test_sparse_align_pose_tolerance(levels, max_level, ctx3, ctx8, oracle):
     fr.close()
 
 
+def test_sparse_align_global_staging(ctx3, oracle):
+    """A problem whose cluster cannot stage its features in shared memory (more than 8 CTAs x (227 KB - 8 KB) / 360 B
+    features) runs from the global staging buffer; the small problem before it checks that the buffer is indexed by the
+    problem's CSR offset."""
+    s = _scene(oracle)
+    g1, d1, T1 = synth.stream_frame(2)
+    g2, _, T2 = synth.stream_frame(5)
+    p1, p2 = oracle.build_pyramid(g1, 3), oracle.build_pyramid(g2, 3)
+    u, v = np.meshgrid(np.arange(4, 636, 5), np.arange(4, 476, 5))
+    dense_px = np.stack([u.ravel() + 0.37, v.ravel() + 0.61], 1)
+    dense_depth = d1[v.ravel(), u.ravel()]
+    n1, n2 = len(s["depth"]), len(dense_depth)
+    assert n2 > 8 * ((227 - 8) * 1024 // 360)
+    has1 = np.ones(n1, np.uint8)
+    has1[::11] = 0
+    has2 = np.ones(n2, np.uint8)
+    fr = ctx3.frames(4)
+    fr.upload(np.stack([s["g1"], s["g2"], g1, g2]))
+    T_ref = np.stack([s["T1"].reshape(-1), T1.reshape(-1)])
+    T, n_meas, _ = fr.sparse_align([0, 2], [1, 3], [0, n1, n1 + n2], np.concatenate([s["px"], dense_px]),
+                                   np.concatenate([s["depth"], dense_depth]), np.concatenate([has1, has2]), T_ref, T_ref)
+    for p, (rp, cp, px, depth, hm, Tr, Tgt) in enumerate(((s["p1"], s["p2"], s["px"], s["depth"], has1, s["T1"], s["T2"]),
+                                                        (p1, p2, dense_px, dense_depth, has2, T1, T2))):
+        wT, wn, _ = oracle.sparse_align(rp, cp, 640, 480, 3, px, depth, hm, Tr, Tr)
+        assert _pose_err(T[p], wT) < 1e-4
+        assert n_meas[p] == wn
+        assert _pose_err(T[p], Tgt) < 2e-3
+    fr.close()
+
+
 def test_align1d_bit_exact(ctx3, oracle):
     """cvutils::Align1D (epipolar 1-D search): u, v, converged flag and h_inv against the oracle."""
     s = _scene(oracle)

@@ -1,5 +1,5 @@
 """Small, bounded inputs for `compute-sanitizer --tool racecheck` on the thread-block-cluster solvers (local_ba2_kernel in its
-lane / warp / CTA-block / scalar solver variants, local_ba_kernel<ceres>, pose_only_kernel).  The parity suite is too slow
+lane / warp / CTA-block / scalar solver variants, local_ba_kernel, pose_only_kernel).  The parity suite is too slow
 under racecheck (the cluster kernels run ~1000x slower), so this drives the same entry points through the C ABI with a few
 LM iterations on small scenes and prints one line per case:
 

@@ -353,269 +353,24 @@ struct SparseArgs {
     double eps;
     int32_t* n_meas_out;        // [n_problems]  (n_meas / 16)
     int32_t* iters_out;         // [n_problems][kMaxLevels] or null
-    // scratch, per feature
-    float* ref_patch;           // [total][16]
-    float* gdx;                 // [total][16]
-    float* gdy;                 // [total][16]
-    double* frame_jac;          // [total][12]
-    uint8_t* visible;           // [total]
-    double* ws;                 // [n_problems][2][kSparseCluster][kNormalTerms + 1]: per-CTA partial sums of an iteration
-    void* feat_scratch;         // second generation: global fall-back of the per-feature staging, feat_stride bytes per problem
-    size_t feat_stride;
+    void* feat_scratch;         // [offsets[n_problems]] SparseFeat: global fall-back of the per-feature staging
 };
 
-// One thread-block CLUSTER per (ref, cur) pair: the normal equations are FP64 (as in the reference) and one SM's FP64
-// pipe bounded the single-CTA version (33 us per Gauss-Newton iteration at 2000 features); the features are strided
-// over the cluster, every CTA publishes its partial sums, one barrier.cluster per iteration, and every CTA then adds the
-// partials in rank order and takes the same solver step on its own replica of the pose.
-constexpr int kSparseCluster = 8;
-constexpr int kSparseThreads = 256;
-constexpr int kNormalTerms = 21 + 6 + 1;  // upper triangle of H, Jres, chi2
-
-__device__ bool ldlt_solve6(const double H[6][6], const double b[6], double x[6]) {
-    double L[6][6], D[6];
-    for (int i = 0; i < 6; ++i)
-        for (int j = 0; j < 6; ++j) L[i][j] = 0;
-    for (int j = 0; j < 6; ++j) {
-        double d = H[j][j];
-        for (int k = 0; k < j; ++k) d -= L[j][k] * L[j][k] * D[k];
-        D[j] = d;
-        if (!(fabs(d) > 0)) return false;
-        L[j][j] = 1;
-        for (int i = j + 1; i < 6; ++i) {
-            double s = H[i][j];
-            for (int k = 0; k < j; ++k) s -= L[i][k] * L[j][k] * D[k];
-            L[i][j] = s / d;
-        }
-    }
-    double y[6];
-    for (int i = 0; i < 6; ++i) {
-        double s = b[i];
-        for (int k = 0; k < i; ++k) s -= L[i][k] * y[k];
-        y[i] = s;
-    }
-    for (int i = 0; i < 6; ++i) y[i] /= D[i];
-    for (int i = 5; i >= 0; --i) {
-        double s = y[i];
-        for (int k = i + 1; k < 6; ++k) s -= L[k][i] * x[k];
-        x[i] = s;
-    }
-    return true;
-}
-
-__global__ void __launch_bounds__(kSparseThreads) sparse_align_kernel(const SparseArgs a) {
-    namespace cg = cooperative_groups;
-    cg::cluster_group cluster = cg::this_cluster();
-    __shared__ double s_red[kSparseThreads / 32][kNormalTerms];
-    __shared__ unsigned long long s_nmeas[kSparseThreads / 32];
-    __shared__ SE3d s_T, s_old;
-    __shared__ int s_flag;        // 0 continue, 1 break (rollback done / converged)
-    __shared__ double s_chi2;     // chi2_ of the solver (persists across levels, NLSSolver_impl.hpp:288-299)
-    __shared__ unsigned long long s_last_nmeas;
-
-    const int rank = (int)cluster.block_rank(), C = (int)cluster.num_blocks();
-    const int prob = blockIdx.x / C, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const int CT = C * kSparseThreads, ct = rank * kSparseThreads + tid;   // cluster-wide thread id
-    const int f0 = a.offsets[prob];
-    const int nf = a.n_feat ? a.n_feat[prob] : a.offsets[prob + 1] - f0;
-    const int f1 = f0 + nf;
-    const long din = a.in_off ? (long)a.in_off[prob] - f0 : 0;   // input index = scratch index + din
-    const Geometry& g = a.g;
-    double* ws = a.ws + (size_t)prob * 2 * kSparseCluster * (kNormalTerms + 1);
-    int slot = 0;
-    if (nf == 0) {  // run(): no features -> returns 0, pose untouched
-        if (rank == 0 && tid == 0) a.n_meas_out[prob] = 0;
-        return;
-    }
-    if (tid == 0) {
-        const SE3d Tref = se3_from_mat(a.T_ref + 12 * (size_t)prob);
-        s_T = se3_mul(se3_from_mat(a.T_cur + 12 * (size_t)prob), se3_inverse(Tref));  // T_cur_from_ref
-        s_chi2 = 1e10;
-        s_last_nmeas = 0;
-    }
-    for (int i = f0 + ct; i < f1; i += CT) a.visible[i] = 0;
-    __syncthreads();
-
-    for (int lvl = a.max_level; lvl >= a.min_level; --lvl) {
-        const LevelImg rim = level_img(a.pyr, a.slot_stride, a.ref_slot[prob], g, lvl);
-        const LevelImg cim = level_img(a.pyr, a.slot_stride, a.cur_slot[prob], g, lvl);
-        const float scale = 1.0f / (float)(1 << lvl);
-        const double focal = (double)(float)((a.cam.fx + a.cam.fy) / 2);  // PinholeCamera::_f is a float
-        const double jscale = focal / (1 << lvl);
-        // precomputeReferencePatches: features that are not cached at this level keep their stale patch with a
-        // zero Jacobian (jacobian_cache_.setZero(); visible_fts_ is never cleared -- kept faithfully)
-        for (int i = f0 + ct; i < f1; i += CT) {   // (per-feature scratch is written and later read by the same thread)
-            for (int k = 0; k < 16; ++k) a.gdx[(size_t)i * 16 + k] = a.gdy[(size_t)i * 16 + k] = 0.f;
-            const float u_ref = (float)(a.px[2 * (i + din)] * scale), v_ref = (float)(a.px[2 * (i + din) + 1] * scale);
-            const int ui = (int)floorf(u_ref), vi = (int)floorf(v_ref);
-            if ((a.has_mp && !a.has_mp[i + din]) || ui - 3 < 0 || vi - 3 < 0 || ui + 3 >= rim.w || vi + 3 >= rim.h) continue;
-            a.visible[i] = 1;
-            const V3d xyz = pixel2camera(a.cam, a.px[2 * (i + din)], a.px[2 * (i + din) + 1], a.depth[i + din]);
-            double* J = a.frame_jac + (size_t)i * 12;
-            const double X = xyz.x, Y = xyz.y, zi = 1. / xyz.z, zi2 = zi * zi;
-            J[0] = -zi; J[1] = 0; J[2] = X * zi2; J[3] = Y * J[2]; J[4] = -(1.0 + X * J[2]); J[5] = Y * zi;
-            J[6] = 0; J[7] = -zi; J[8] = Y * zi2; J[9] = 1.0 + Y * J[8]; J[10] = -J[3]; J[11] = -X * zi;
-            const float su = u_ref - (float)ui, sv = v_ref - (float)vi;
-            const float wtl = (float)((1.0 - su) * (1.0 - sv)), wtr = (float)(su * (1.0 - sv)), wbl = (float)((1.0 - su) * sv),
-                        wbr = su * sv;
-            const int st = rim.pitch;
-            int pc = 0;
-            for (int y = 0; y < 4; ++y) {
-                const uint8_t* p = rim.d + (size_t)(vi + y - 2) * st + (ui - 2);
-                for (int xx = 0; xx < 4; ++xx, ++p, ++pc) {
-                    a.ref_patch[(size_t)i * 16 + pc] = wtl * (float)p[0] + wtr * (float)p[1] + wbl * (float)p[st] + wbr * (float)p[st + 1];
-                    a.gdx[(size_t)i * 16 + pc] =
-                        0.5f * ((wtl * (float)p[1] + wtr * (float)p[2] + wbl * (float)p[st + 1] + wbr * (float)p[st + 2]) -
-                                (wtl * (float)p[-1] + wtr * (float)p[0] + wbl * (float)p[st - 1] + wbr * (float)p[st]));
-                    a.gdy[(size_t)i * 16 + pc] =
-                        0.5f * ((wtl * (float)p[st] + wtr * (float)p[1 + st] + wbl * (float)p[st * 2] + wbr * (float)p[st * 2 + 1]) -
-                                (wtl * (float)p[-st] + wtr * (float)p[1 - st] + wbl * (float)p[0] + wbr * (float)p[1]));
-                }
-            }
-        }
-        if (tid == 0) {
-            s_old = s_T;
-            s_flag = 0;
-        }
-        __syncthreads();
-
-        int it = 0;
-        for (it = 0; it < a.n_iter; ++it) {
-            const SE3d T = s_T;
-            double acc[kNormalTerms];
-#pragma unroll
-            for (int k = 0; k < kNormalTerms; ++k) acc[k] = 0.0;
-            unsigned long long nm = 0;
-            for (int i = f0 + ct; i < f1; i += CT) {
-                if (!a.visible[i]) continue;
-                const V3d xyz_ref = pixel2camera(a.cam, a.px[2 * (i + din)], a.px[2 * (i + din) + 1], a.depth[i + din]);
-                const V3d xyz_cur = transform(T, xyz_ref);
-                double pu, pv;
-                camera2pixel(a.cam, xyz_cur, &pu, &pv);
-                const float u_cur = (float)pu * scale, v_cur = (float)pv * scale;
-                const int ui = (int)floorf(u_cur), vi = (int)floorf(v_cur);
-                if (ui < 0 || vi < 0 || ui - 3 < 0 || vi - 3 < 0 || ui + 3 >= cim.w || vi + 3 >= cim.h) continue;
-                const float su = u_cur - (float)ui, sv = v_cur - (float)vi;
-                const float wtl = (float)((1.0 - su) * (1.0 - sv)), wtr = (float)(su * (1.0 - sv)),
-                            wbl = (float)((1.0 - su) * sv), wbr = su * sv;
-                const double* FJ = a.frame_jac + (size_t)i * 12;
-                const int st = cim.pitch;
-                int pc = 0;
-                for (int y = 0; y < 4; ++y) {
-                    const uint8_t* p = cim.d + (size_t)(vi + y - 2) * st + (ui - 2);
-                    for (int xx = 0; xx < 4; ++xx, ++pc, ++p) {
-                        const float inten = wtl * (float)p[0] + wtr * (float)p[1] + wbl * (float)p[st] + wbr * (float)p[st + 1];
-                        const float res = inten - a.ref_patch[(size_t)i * 16 + pc];
-                        acc[27] += (double)(res * res);
-                        ++nm;
-                        const float dx = a.gdx[(size_t)i * 16 + pc], dy = a.gdy[(size_t)i * 16 + pc];
-                        double J[6];
-#pragma unroll
-                        for (int k = 0; k < 6; ++k) J[k] = (dx * FJ[k] + dy * FJ[6 + k]) * jscale;
-                        int t = 0;
-#pragma unroll
-                        for (int r = 0; r < 6; ++r) {
-#pragma unroll
-                            for (int c = r; c < 6; ++c, ++t) acc[t] = fma(J[r], J[c], acc[t]);   // explicit FMA: the file is built with -fmad=false
-                        }
-#pragma unroll
-                        for (int k = 0; k < 6; ++k) acc[21 + k] = fma(-J[k], (double)res, acc[21 + k]);
-                    }
-                }
-            }
-            // block reduction (warp shuffles, then shared memory)
-#pragma unroll
-            for (int k = 0; k < kNormalTerms; ++k) {
-                double v = acc[k];
-#pragma unroll
-                for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xFFFFFFFFu, v, o);
-                if (lane == 0) s_red[warp][k] = v;
-            }
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1) nm += __shfl_down_sync(0xFFFFFFFFu, nm, o);
-            if (lane == 0) s_nmeas[warp] = nm;
-            __syncthreads();
-            // CTA partials -> workspace, barrier.cluster, then every CTA adds the partials of all ranks in rank order
-            double* my = ws + ((size_t)slot * kSparseCluster + rank) * (kNormalTerms + 1);
-            if (tid <= kNormalTerms) {
-                double v = 0;
-                if (tid < kNormalTerms) {
-                    for (int w = 0; w < kSparseThreads / 32; ++w) v += s_red[w][tid];
-                } else {
-                    unsigned long long n = 0;
-                    for (int w = 0; w < kSparseThreads / 32; ++w) n += s_nmeas[w];
-                    v = (double)n;   // < 2^53: exact
-                }
-                my[tid] = v;
-            }
-            cluster.sync();
-            if (tid == 0) {
-                double tot[kNormalTerms];
-                unsigned long long n_meas = 0;
-                for (int k = 0; k < kNormalTerms; ++k) tot[k] = 0;
-                for (int r = 0; r < C; ++r) {
-                    const double* pr = ws + ((size_t)slot * kSparseCluster + r) * (kNormalTerms + 1);
-                    for (int k = 0; k < kNormalTerms; ++k) tot[k] += __ldcg(pr + k);
-                    n_meas += (unsigned long long)__ldcg(pr + kNormalTerms);
-                }
-                s_last_nmeas = n_meas;
-                double H[6][6], b[6], x[6];
-                int t = 0;
-                for (int r = 0; r < 6; ++r)
-                    for (int c = r; c < 6; ++c) {
-                        H[r][c] = H[c][r] = tot[t++];
-                    }
-                for (int k = 0; k < 6; ++k) b[k] = tot[21 + k];
-                // computeResiduals returns (float chi2) / n_meas
-                const double new_chi2 = (double)((float)tot[27] / (float)n_meas);
-                bool stop = !ldlt_solve6(H, b, x) || isnan(x[0]);
-                if ((it > 0 && new_chi2 > s_chi2) || stop) {
-                    s_T = s_old;  // rollback
-                    s_flag = 1;
-                } else {
-                    double mx[6];
-                    for (int k = 0; k < 6; ++k) mx[k] = -x[k];
-                    const SE3d Tn = se3_mul(s_T, se3_exp(mx));  // update(): T_new = T_old * exp(-x)
-                    s_old = s_T;
-                    s_T = Tn;
-                    s_chi2 = new_chi2;
-                    double nmx = -1;
-                    for (int k = 0; k < 6; ++k) nmx = fabs(x[k]) > nmx ? fabs(x[k]) : nmx;
-                    if (nmx <= a.eps) s_flag = 1;
-                }
-            }
-            slot ^= 1;
-            __syncthreads();
-            if (s_flag) break;
-        }
-        if (rank == 0 && tid == 0 && a.iters_out) a.iters_out[prob * kMaxLevels + lvl] = it;
-        __syncthreads();
-    }
-    cluster.sync();   // no CTA may exit while another still reads its partials
-    if (rank == 0 && tid == 0) {
-        const SE3d Tref = se3_from_mat(a.T_ref + 12 * (size_t)prob);
-        se3_to_mat(se3_mul(s_T, Tref), a.T_cur + 12 * (size_t)prob);
-        a.n_meas_out[prob] = (int32_t)(s_last_nmeas / 16);
-    }
-}
-
-
-// ---- SparseImgAlign, second generation (the tracking engine's batches) -------------------------------------------------
-// Same Gauss-Newton as sparse_align_kernel, reorganised around what ncu showed on it (one third of the time in the
-// single-thread solve + cluster barrier, the rest a per-thread chain of 16 pixels x 27 FP64 FMAs):
+// One thread-block CLUSTER per (ref, cur) pair: the normal equations are FP64 (as in the reference), and one SM's FP64
+// pipe would bound a single CTA.  The Gauss-Newton of the reference is reorganised around the FP64 work:
 //   * J_px = (dx FJ0 + dy FJ1) * s  (FJ0/FJ1 = the two 6-vectors of the feature, dx/dy = reference gradients, s = f / 2^level),
 //     so  sum_px J J^T = s^2 (Gxx FJ0 FJ0^T + Gxy (FJ0 FJ1^T + FJ1 FJ0^T) + Gyy FJ1 FJ1^T)  with per-feature constants
 //     G = sum_px (dx^2, dx dy, dy^2), and  sum_px J res = s (FJ0 sum dx res + FJ1 sum dy res): an iteration costs 3 FP64 FMAs per
 //     pixel + ~75 per feature instead of 27 per pixel;
 //   * the features are partitioned over the CTAs of the cluster and staged in shared memory (reference patch, gradients, FJ,
-//     G, camera-frame point); 4 lanes share a feature (one patch row each);
+//     G, camera-frame point), or in global memory when a CTA's share does not fit; 4 lanes share a feature (one patch row each);
 //   * per-iteration partial sums are exchanged through distributed shared memory (one cluster barrier), every CTA adds them
 //     in rank order and takes the same step (LDL^T with hardware-seeded reciprocals).
-// Results agree with sparse_align_kernel to rounding (different summation order): the engine's trajectory parity test bounds it.
-constexpr int kSA2Threads = 256;
-constexpr int kSA2Terms = 21 + 6 + 1;   // H upper triangle, Jres, chi2 (+ the measurement count in a separate integer)
+constexpr int kSparseThreads = 256;
+constexpr int kSparseCluster = 8;          // CTAs per problem of ygzb_sparse_align (the tracker chooses its own)
+constexpr int kNormalTerms = 21 + 6 + 1;   // H upper triangle, Jres, chi2 (+ the measurement count in a separate integer)
 
-struct SA2Feat {           // 4-byte fields first: arrays of structs in shared memory, one per feature of the CTA
+struct SparseFeat {           // 4-byte fields first: arrays of structs in shared memory, one per feature of the CTA
     float patch[16], gdx[16], gdy[16];
     double FJ[12];
     double G[3];
@@ -626,7 +381,7 @@ struct SA2Feat {           // 4-byte fields first: arrays of structs in shared m
     int pad;
 };
 
-__device__ __forceinline__ double sa2_rcp(double x) {
+__device__ __forceinline__ double rcp_f64(double x) {
     double r;
     asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(r) : "d"(x));
     r = fma(r, fma(-x, r, 1.0), r);
@@ -634,14 +389,14 @@ __device__ __forceinline__ double sa2_rcp(double x) {
     return r;
 }
 
-__device__ bool ldlt_solve6_fast(const double H[6][6], const double b[6], double x[6]) {
+__device__ bool ldlt_solve6(const double H[6][6], const double b[6], double x[6]) {
     double L[6][6], D[6], rD[6];
     for (int j = 0; j < 6; ++j) {
         double d = H[j][j];
         for (int k = 0; k < j; ++k) d -= L[j][k] * L[j][k] * D[k];
         D[j] = d;
         if (!(fabs(d) > 0)) return false;
-        rD[j] = sa2_rcp(fabs(d));
+        rD[j] = rcp_f64(fabs(d));
         if (d < 0) rD[j] = -rD[j];
         L[j][j] = 1;
         for (int i = j + 1; i < 6; ++i) {
@@ -665,13 +420,13 @@ __device__ bool ldlt_solve6_fast(const double H[6][6], const double b[6], double
     return true;
 }
 
-__global__ void __launch_bounds__(kSA2Threads) sparse_align2_kernel(const SparseArgs a, int feat_cap /* features per CTA that fit shared memory */) {
+__global__ void __launch_bounds__(kSparseThreads) sparse_align_kernel(const SparseArgs a, int feat_cap /* features per CTA that fit shared memory */) {
     namespace cg = cooperative_groups;
     cg::cluster_group cluster = cg::this_cluster();
     extern __shared__ __align__(16) unsigned char s_raw[];
-    __shared__ double s_red[kSA2Threads / 32][kSA2Terms];
-    __shared__ unsigned s_nm[kSA2Threads / 32];
-    __shared__ double s_part[2][kSA2Terms + 1];   // this CTA's partial sums of an iteration (double buffered), [kSA2Terms] = count
+    __shared__ double s_red[kSparseThreads / 32][kNormalTerms];
+    __shared__ unsigned s_nm[kSparseThreads / 32];
+    __shared__ double s_part[2][kNormalTerms + 1];   // this CTA's partial sums of an iteration (double buffered), [kNormalTerms] = count
     __shared__ SE3d s_T, s_old;
     __shared__ double s_Tm[12];
     __shared__ int s_flag;
@@ -691,21 +446,20 @@ __global__ void __launch_bounds__(kSA2Threads) sparse_align2_kernel(const Sparse
     // this CTA's features: a contiguous share, staged in shared memory (the launcher sizes the cluster so that it fits)
     const int per = (nf + C - 1) / C;
     const int j_lo = min(nf, rank * per), nl = min(nf, j_lo + per) - j_lo;
-    SA2Feat* F = nl <= feat_cap ? reinterpret_cast<SA2Feat*>(s_raw)
-                                : reinterpret_cast<SA2Feat*>(static_cast<unsigned char*>(a.feat_scratch) + (size_t)prob * a.feat_stride) + j_lo;
+    SparseFeat* F = nl <= feat_cap ? reinterpret_cast<SparseFeat*>(s_raw) : static_cast<SparseFeat*>(a.feat_scratch) + f0 + j_lo;
     if (tid == 0) {
         const SE3d Tref = se3_from_mat(a.T_ref + 12 * (size_t)prob);
         s_T = se3_mul(se3_from_mat(a.T_cur + 12 * (size_t)prob), se3_inverse(Tref));
         s_chi2 = 1e10;
         s_last_nmeas = 0;
     }
-    for (int j = tid; j < nl; j += kSA2Threads) {
-        SA2Feat& ft = F[j];
+    for (int j = tid; j < nl; j += kSparseThreads) {
+        SparseFeat& ft = F[j];
         const long gi = f0 + j_lo + j + din;
         ft.state = 0;
         const V3d xyz = pixel2camera(a.cam, a.px[2 * gi], a.px[2 * gi + 1], a.depth[gi]);
         ft.xyz[0] = xyz.x; ft.xyz[1] = xyz.y; ft.xyz[2] = xyz.z;
-        for (int k = 0; k < 16; ++k) ft.patch[k] = 0.f;   // (the API path clears its patch scratch before the launch)
+        for (int k = 0; k < 16; ++k) ft.patch[k] = 0.f;
     }
     __syncthreads();
     int slot = 0;
@@ -717,8 +471,8 @@ __global__ void __launch_bounds__(kSA2Threads) sparse_align2_kernel(const Sparse
         const double focal = (double)(float)((a.cam.fx + a.cam.fy) / 2);  // PinholeCamera::_f is a float
         const double jscale = focal / (1 << lvl);
         // precomputeReferencePatches (features that are not cached at this level keep their stale patch with a zero Jacobian)
-        for (int j = tid; j < nl; j += kSA2Threads) {
-            SA2Feat& ft = F[j];
+        for (int j = tid; j < nl; j += kSparseThreads) {
+            SparseFeat& ft = F[j];
             const long gi = f0 + j_lo + j + din;
             for (int k = 0; k < 16; ++k) ft.gdx[k] = ft.gdy[k] = 0.f;
             ft.G[0] = ft.G[1] = ft.G[2] = 0.0;
@@ -762,8 +516,8 @@ __global__ void __launch_bounds__(kSA2Threads) sparse_align2_kernel(const Sparse
         int it = 0;
         for (it = 0; it < a.n_iter; ++it) {
             // phase A: projection of every visible feature at the current pose
-            for (int j = tid; j < nl; j += kSA2Threads) {
-                SA2Feat& ft = F[j];
+            for (int j = tid; j < nl; j += kSparseThreads) {
+                SparseFeat& ft = F[j];
                 if (!(ft.state & 1)) continue;
                 ft.state &= ~2;
                 const double x = s_Tm[0] * ft.xyz[0] + s_Tm[1] * ft.xyz[1] + s_Tm[2] * ft.xyz[2] + s_Tm[3];
@@ -779,12 +533,12 @@ __global__ void __launch_bounds__(kSA2Threads) sparse_align2_kernel(const Sparse
             }
             __syncthreads();
             // phase B: (feature, patch row) items over the threads
-            double acc[kSA2Terms];
+            double acc[kNormalTerms];
 #pragma unroll
-            for (int k = 0; k < kSA2Terms; ++k) acc[k] = 0.0;
+            for (int k = 0; k < kNormalTerms; ++k) acc[k] = 0.0;
             unsigned nm = 0;
-            for (int item = tid; item < nl * 4; item += kSA2Threads) {
-                const SA2Feat& ft = F[item >> 2];
+            for (int item = tid; item < nl * 4; item += kSparseThreads) {
+                const SparseFeat& ft = F[item >> 2];
                 if ((ft.state & 3) != 3) continue;
                 const int y = item & 3;
                 const float su = ft.u - (float)ft.ui, sv = ft.v - (float)ft.vi;
@@ -815,7 +569,7 @@ __global__ void __launch_bounds__(kSA2Threads) sparse_align2_kernel(const Sparse
                 }
             }
 #pragma unroll
-            for (int k = 0; k < kSA2Terms; ++k) {
+            for (int k = 0; k < kNormalTerms; ++k) {
                 double v = acc[k];
 #pragma unroll
                 for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xFFFFFFFFu, v, o);
@@ -825,26 +579,26 @@ __global__ void __launch_bounds__(kSA2Threads) sparse_align2_kernel(const Sparse
             for (int o = 16; o > 0; o >>= 1) nm += __shfl_down_sync(0xFFFFFFFFu, nm, o);
             if (lane == 0) s_nm[warp] = nm;
             __syncthreads();
-            if (tid <= kSA2Terms) {
+            if (tid <= kNormalTerms) {
                 double v = 0;
-                if (tid < kSA2Terms) {
-                    for (int w = 0; w < kSA2Threads / 32; ++w) v += s_red[w][tid];
+                if (tid < kNormalTerms) {
+                    for (int w = 0; w < kSparseThreads / 32; ++w) v += s_red[w][tid];
                 } else {
                     unsigned n = 0;
-                    for (int w = 0; w < kSA2Threads / 32; ++w) n += s_nm[w];
+                    for (int w = 0; w < kSparseThreads / 32; ++w) n += s_nm[w];
                     v = (double)n;
                 }
                 s_part[slot][tid] = v;
             }
             cluster.sync();
             if (tid == 0) {
-                double tot[kSA2Terms];
+                double tot[kNormalTerms];
                 unsigned long long n_meas = 0;
-                for (int k = 0; k < kSA2Terms; ++k) tot[k] = 0;
+                for (int k = 0; k < kNormalTerms; ++k) tot[k] = 0;
                 for (int r = 0; r < C; ++r) {
                     const double* pr = cluster.map_shared_rank(&s_part[slot][0], r);
-                    for (int k = 0; k < kSA2Terms; ++k) tot[k] += pr[k];
-                    n_meas += (unsigned long long)pr[kSA2Terms];
+                    for (int k = 0; k < kNormalTerms; ++k) tot[k] += pr[k];
+                    n_meas += (unsigned long long)pr[kNormalTerms];
                 }
                 s_last_nmeas = n_meas;
                 double H[6][6], b[6], x[6];
@@ -853,7 +607,7 @@ __global__ void __launch_bounds__(kSA2Threads) sparse_align2_kernel(const Sparse
                     for (int c = r; c < 6; ++c) H[r][c] = H[c][r] = tot[t++];
                 for (int k = 0; k < 6; ++k) b[k] = tot[21 + k];
                 const double new_chi2 = (double)((float)tot[27] / (float)n_meas);
-                bool stop = !ldlt_solve6_fast(H, b, x) || isnan(x[0]);
+                bool stop = !ldlt_solve6(H, b, x) || isnan(x[0]);
                 if ((it > 0 && new_chi2 > s_chi2) || stop) {
                     s_T = s_old;  // rollback
                     s_flag = 1;
@@ -1047,10 +801,46 @@ __global__ void __launch_bounds__(1024) track_compact_kernel(TrackStore st, Trac
     if (tid == 0) b.c_cnt[j] = s_carry;
 }
 
+// One cluster of `cluster` CTAs per problem.  A CTA stages its share of a problem's features, at most
+// ceil(max_feat / cluster), in dynamic shared memory, or in a.feat_scratch when that share exceeds what a CTA can opt in to.
+// Fills the frame fields of `a` (pyramids, geometry, camera) from f.
+int launch_sparse_align_kernel(ygzb_frames* f, SparseArgs a, int n_problems, int max_feat, int cluster) {
+    ygzb_ctx* ctx = f->ctx;
+    a.pyr = f->d_pyr;
+    a.slot_stride = ctx->slot_stride;
+    a.g = ctx->geo;
+    a.cam = CamF{ctx->prm.fx, ctx->prm.fy, ctx->prm.cx, ctx->prm.cy};
+    static std::once_flag once;
+    static int max_dyn = 0;
+    std::call_once(once, [] {
+        int dev = 0, optin = 0;
+        cudaGetDevice(&dev);
+        cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
+        max_dyn = optin - 8 * 1024;   // the kernel's static arrays
+        cudaFuncSetAttribute(sparse_align_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, max_dyn);
+    });
+    const int feat_cap = max_dyn / (int)sizeof(SparseFeat);
+    cudaLaunchConfig_t cfg{};
+    cfg.gridDim = dim3((unsigned)(n_problems * cluster));
+    cfg.blockDim = dim3(kSparseThreads);
+    cfg.dynamicSmemBytes = (size_t)std::min(feat_cap, (max_feat + cluster - 1) / cluster) * sizeof(SparseFeat);
+    cfg.stream = ctx->stream;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeClusterDimension;
+    attr[0].val.clusterDim.x = cluster;
+    attr[0].val.clusterDim.y = 1;
+    attr[0].val.clusterDim.z = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    ProfScope ps(ctx, kStageSparseAlign);
+    YGZB_CUDA(ctx, cudaLaunchKernelEx(&cfg, sparse_align_kernel, a, feat_cap));
+    YGZB_LAUNCHED(ctx);
+    return YGZB_OK;
+}
+
 }  // namespace
 
-size_t sparse_align2_scratch_bytes(int n_problems, int cells) { return (size_t)n_problems * cells * sizeof(SA2Feat); }
-size_t sparse_align_ws_doubles(int n_problems) { return (size_t)n_problems * 2 * kSparseCluster * (kNormalTerms + 1); }
+size_t sparse_align_scratch_bytes(size_t n_features) { return n_features * sizeof(SparseFeat); }
 
 int launch_align2d(ygzb_frames* f, int n, const int32_t* d_slot, const uint8_t* d_level, const uint8_t* d_ref_border,
                    const uint8_t* d_ref, int n_iter, double* d_uv, uint8_t* d_ok) {
@@ -1089,22 +879,14 @@ int launch_project_align(ygzb_frames* f, int n, const int32_t* d_ref_slot, const
 }
 
 int launch_sparse_align(ygzb_frames* f, int n_problems, const int32_t* d_ref_slot, const int32_t* d_cur_slot,
-                        const int32_t* d_offsets, const double* d_px, const double* d_depth, const uint8_t* d_has_mp,
+                        const int32_t* d_offsets, int max_feat, const double* d_px, const double* d_depth, const uint8_t* d_has_mp,
                         const double* d_T_ref, double* d_T_cur, int max_level, int min_level, int n_iter, double eps,
-                        int32_t* d_n_meas, int32_t* d_iters, float* d_ref_patch, float* d_gdx, float* d_gdy, double* d_frame_jac,
-                        uint8_t* d_visible, double* d_ws) {
-    ygzb_ctx* ctx = f->ctx;
+                        int32_t* d_n_meas, int32_t* d_iters, void* d_feat_scratch) {
     if (n_problems <= 0) return YGZB_OK;
-    SparseArgs a;
-    a.pyr = f->d_pyr;
-    a.slot_stride = ctx->slot_stride;
-    a.g = ctx->geo;
-    a.cam = CamF{ctx->prm.fx, ctx->prm.fy, ctx->prm.cx, ctx->prm.cy};
+    SparseArgs a{};
     a.ref_slot = d_ref_slot;
     a.cur_slot = d_cur_slot;
     a.offsets = d_offsets;
-    a.in_off = nullptr;
-    a.n_feat = nullptr;
     a.px = d_px;
     a.depth = d_depth;
     a.has_mp = d_has_mp;
@@ -1116,32 +898,9 @@ int launch_sparse_align(ygzb_frames* f, int n_problems, const int32_t* d_ref_slo
     a.eps = eps;
     a.n_meas_out = d_n_meas;
     a.iters_out = d_iters;
-    a.ref_patch = d_ref_patch;
-    a.gdx = d_gdx;
-    a.gdy = d_gdy;
-    a.frame_jac = d_frame_jac;
-    a.visible = d_visible;
-    a.ws = d_ws;
-    a.feat_scratch = nullptr;
-    a.feat_stride = 0;
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3((unsigned)(n_problems * kSparseCluster));
-    cfg.blockDim = dim3(kSparseThreads);
-    cfg.dynamicSmemBytes = 0;
-    cfg.stream = ctx->stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = kSparseCluster;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    ProfScope ps(ctx, kStageSparseAlign);
-    YGZB_CUDA(ctx, cudaLaunchKernelEx(&cfg, sparse_align_kernel, a));
-    YGZB_LAUNCHED(ctx);
-    return YGZB_OK;
+    a.feat_scratch = d_feat_scratch;
+    return launch_sparse_align_kernel(f, a, n_problems, max_feat, kSparseCluster);
 }
-
 
 // Tracking chain of a batch, part 1 (on whatever stream ctx->stream currently is: the tracker points it at its second
 // stream): prep -> sparse alignment relative to the reference key-frame.  Needs the key-frame's features, not its pose.
@@ -1153,76 +912,25 @@ int launch_track_chain_front(ygzb_frames* f, const TrackStore& st, const TrackBa
         track_prep_kernel<<<(b.J + 127) / 128, 128, 0, ctx->stream>>>(st, b);
         YGZB_LAUNCHED(ctx);
     }
-    if (getenv("YGZB_SPARSE_GEN1"))   // (the second-generation kernel keeps its patches in shared memory)
-        YGZB_CUDA(ctx, cudaMemsetAsync(b.ref_patch, 0, (size_t)b.J * st.cells * 16 * sizeof(float), ctx->stream));
-    {
-        SparseArgs a;
-        a.pyr = f->d_pyr;
-        a.slot_stride = ctx->slot_stride;
-        a.g = ctx->geo;
-        a.cam = CamF{ctx->prm.fx, ctx->prm.fy, ctx->prm.cx, ctx->prm.cy};
-        a.ref_slot = b.ref_slot;
-        a.cur_slot = b.cur_slot;
-        a.offsets = b.offsets;
-        a.in_off = b.in_off;
-        a.n_feat = b.n_feat;
-        a.px = st.kf_px;
-        a.depth = st.kf_depth;
-        a.has_mp = nullptr;            // every feature of a key-frame has its map point (depth-initialised)
-        a.T_ref = b.T_ref;
-        a.T_cur = b.T_cur;
-        a.max_level = 2;               // Matcher's SparseImgAlign(2, 0, 30, GaussNewton) (Matcher.cpp:18)
-        a.min_level = 0;
-        a.n_iter = 30;
-        a.eps = 1e-6;
-        a.n_meas_out = b.n_meas;
-        a.iters_out = nullptr;
-        a.ref_patch = b.ref_patch;
-        a.gdx = b.gdx;
-        a.gdy = b.gdy;
-        a.frame_jac = b.frame_jac;
-        a.visible = b.visible;
-        a.ws = b.sparse_ws;
-        // second-generation kernel: the features of a problem are staged in the shared memory of its cluster
-        static std::once_flag once;
-        static int max_dyn = 0;
-        std::call_once(once, [&] {
-            int dev = 0, optin = 0;
-            cudaGetDevice(&dev);
-            cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
-            max_dyn = optin - 8 * 1024;   // the kernel's static arrays
-            cudaFuncSetAttribute(sparse_align2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, max_dyn);
-        });
-        const int feat_cap = max_dyn / (int)sizeof(SA2Feat);
-        const int cl = sparse_cluster;
-        const size_t dyn = (size_t)std::min(feat_cap, (st.cells + cl - 1) / cl) * sizeof(SA2Feat);
-        a.feat_scratch = b.sa2_scratch;          // used only by a CTA whose share of the features exceeds its shared memory
-        a.feat_stride = (size_t)st.cells * sizeof(SA2Feat);
-        cudaLaunchConfig_t cfg{};
-        cfg.gridDim = dim3((unsigned)(b.J * cl));
-        cfg.blockDim = dim3(kSA2Threads);
-        cfg.dynamicSmemBytes = dyn;
-        cfg.stream = ctx->stream;
-        cudaLaunchAttribute attr[1];
-        attr[0].id = cudaLaunchAttributeClusterDimension;
-        attr[0].val.clusterDim.x = cl;
-        attr[0].val.clusterDim.y = 1;
-        attr[0].val.clusterDim.z = 1;
-        cfg.attrs = attr;
-        cfg.numAttrs = 1;
-        ProfScope ps(ctx, kStageSparseAlign);
-        if (getenv("YGZB_SPARSE_GEN1")) {
-            cfg.gridDim = dim3((unsigned)(b.J * sparse_cluster));
-            cfg.blockDim = dim3(kSparseThreads);
-            cfg.dynamicSmemBytes = 0;
-            attr[0].val.clusterDim.x = sparse_cluster;
-            YGZB_CUDA(ctx, cudaLaunchKernelEx(&cfg, sparse_align_kernel, a));
-        } else {
-            YGZB_CUDA(ctx, cudaLaunchKernelEx(&cfg, sparse_align2_kernel, a, feat_cap));
-        }
-        YGZB_LAUNCHED(ctx);
-    }
-    return YGZB_OK;
+    SparseArgs a{};
+    a.ref_slot = b.ref_slot;
+    a.cur_slot = b.cur_slot;
+    a.offsets = b.offsets;
+    a.in_off = b.in_off;
+    a.n_feat = b.n_feat;
+    a.px = st.kf_px;
+    a.depth = st.kf_depth;
+    a.has_mp = nullptr;            // every feature of a key-frame has its map point (depth-initialised)
+    a.T_ref = b.T_ref;
+    a.T_cur = b.T_cur;
+    a.max_level = 2;               // Matcher's SparseImgAlign(2, 0, 30, GaussNewton) (Matcher.cpp:18)
+    a.min_level = 0;
+    a.n_iter = 30;
+    a.eps = 1e-6;
+    a.n_meas_out = b.n_meas;
+    a.iters_out = nullptr;
+    a.feat_scratch = b.feat_scratch;
+    return launch_sparse_align_kernel(f, a, b.J, st.cells, sparse_cluster);
 }
 
 // part 2 (main stream, behind a local BA in flight): key-frame pose applied -> motion check / relative poses -> candidate

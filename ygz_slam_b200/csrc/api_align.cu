@@ -176,11 +176,12 @@ int ygzb_sparse_align(ygzb_frames* f, int n_problems, const int32_t* ref_slot, c
     TRY(check_offsets(ctx, offsets, n_problems, "offsets"));
     const size_t P = (size_t)n_problems, T = (size_t)offsets[n_problems];
     if (T && (!px || !depth || !has_mappoint)) return YGZB_ERR_INVALID;
+    int max_feat = 0;
+    for (int p = 0; p < n_problems; ++p) max_feat = std::max(max_feat, offsets[p + 1] - offsets[p]);
     Carver sz(nullptr);
     sz.take<int32_t>(2 * P); sz.take<int32_t>(P + 1); sz.take<double>(2 * T); sz.take<double>(T); sz.take<uint8_t>(T);
     sz.take<double>(12 * P); sz.take<double>(12 * P); sz.take<int32_t>(P); sz.take<int32_t>(P * kMaxLevels);
-    sz.take<float>(16 * T); sz.take<float>(16 * T); sz.take<float>(16 * T); sz.take<double>(12 * T); sz.take<uint8_t>(T);
-    sz.take<double>(sparse_align_ws_doubles(n_problems));
+    sz.take<uint8_t>(sparse_align_scratch_bytes(T));
     void* buf = dev_scratch(ctx, 6, sz.bytes());
     if (!buf) return YGZB_ERR_CUDA;
     Carver c(buf);
@@ -193,12 +194,7 @@ int ygzb_sparse_align(ygzb_frames* f, int n_problems, const int32_t* ref_slot, c
     double* d_Tcur = c.take<double>(12 * P);
     int32_t* d_nmeas = c.take<int32_t>(P);
     int32_t* d_iters = c.take<int32_t>(P * kMaxLevels);
-    float* d_patch = c.take<float>(16 * T);
-    float* d_gdx = c.take<float>(16 * T);
-    float* d_gdy = c.take<float>(16 * T);
-    double* d_fj = c.take<double>(12 * T);
-    uint8_t* d_vis = c.take<uint8_t>(T);
-    double* d_ws = c.take<double>(sparse_align_ws_doubles(n_problems));
+    void* d_feat = c.take<uint8_t>(sparse_align_scratch_bytes(T));
     {   // the inputs are the first seven sub-buffers of `buf`: one pinned staging copy instead of eight pageable ones
         const size_t in_bytes = (size_t)((uint8_t*)(d_Tcur + 12 * P) - (uint8_t*)buf);
         uint8_t* stage = (uint8_t*)host_scratch(ctx, 1, in_bytes);
@@ -218,9 +214,8 @@ int ygzb_sparse_align(ygzb_frames* f, int n_problems, const int32_t* ref_slot, c
         YGZB_CUDA(ctx, cudaMemcpyAsync(buf, stage, in_bytes, cudaMemcpyHostToDevice, ctx->stream));
     }
     YGZB_CUDA(ctx, cudaMemsetAsync(d_iters, 0, P * kMaxLevels * sizeof(int32_t), ctx->stream));
-    YGZB_CUDA(ctx, cudaMemsetAsync(d_patch, 0, 16 * T * sizeof(float), ctx->stream));
-    TRY(launch_sparse_align(f, n_problems, d_slots, d_slots + P, d_off, d_px, d_depth, d_mp, d_Tref, d_Tcur, max_level, min_level,
-                            n_iter, eps, d_nmeas, d_iters, d_patch, d_gdx, d_gdy, d_fj, d_vis, d_ws));
+    TRY(launch_sparse_align(f, n_problems, d_slots, d_slots + P, d_off, max_feat, d_px, d_depth, d_mp, d_Tref, d_Tcur, max_level,
+                            min_level, n_iter, eps, d_nmeas, d_iters, d_feat));
     TRY(d2h(ctx, T_cw_cur, d_Tcur, 12 * P));
     TRY(d2h(ctx, n_meas, d_nmeas, P));
     if (iters_per_level) TRY(d2h(ctx, iters_per_level, d_iters, P * kMaxLevels));

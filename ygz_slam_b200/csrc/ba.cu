@@ -1,18 +1,17 @@
-// ba.cu -- local bundle adjustment (g2o-style Levenberg + Schur complement) and pose-only refinement
-// (Ceres-style trust-region LM), each as ONE persistent CTA per problem: the whole optimisation loop runs
-// on the device, the host sees one launch per batch of problems.
+// ba.cu -- local bundle adjustment of the Ceres twin (trust-region LM + Schur complement) and pose-only refinement
+// (Ceres-style trust-region LM), each as ONE persistent CTA cluster per problem: the whole optimisation loop runs
+// on the device, the host sees one launch per batch of problems.  ba::LocalBAG2O runs in ba2.cu; its C ABI
+// marshalling is here.
 //
 // Replaces:
-//   ba::LocalBAG2O                   reference src/Algorithm/BA.cpp:386-543
-//   VertexSE3Sophus::oplusImpl       reference include/ygz/G2oTypes.h:38-45
-//   EdgeSophusSE3ProjectXYZ          reference include/ygz/G2oTypes.h:84-132 (computeError, linearizeOplus)
+//   ba::LocalBA, ba::TwoViewBACeres  reference src/Algorithm/BA.cpp:324-385, 11-89
 //   ba::OptimizeCurrentPoseOnly      reference src/Algorithm/BA.cpp:188-264
 //   CeresReprojectionErrorPoseOnly   reference include/ygz/Ceres/CeresReprojectionErrorPoseOnly.h:27-58
 // g2o / Ceres themselves are outside the reference tree: the optimiser logic follows the published
 // algorithms as pinned in oracle/ba.cpp (SURVEY.md appendix A.3 / A.4).
 //
 // Local BA, per LM trial (C4: 10 keyframes, 2000 landmarks, ~8000 observations):
-//   linearise      thread per observation : error, Huber weight, 2x3 / 2x6 Jacobians        (~300 FLOP/obs)
+//   linearise      thread per observation : error, Huber weight, 2x3 / 2x6 Jacobians by forward-mode jets
 //   Hll, bl        thread per landmark    : sum over its observations (CSR by landmark)
 //   Hpp, bp        warp per free pose     : warp-shuffle reduction of J^T J (21+6 terms) over its observations
 //   Schur S, b_s   warp per 6x6 block pair: S(f1,f2) -= Hpl Hll^-1 Hpl^T over the landmarks seen by both poses,
@@ -47,7 +46,7 @@ constexpr int kMaxPoses = 64;
 struct BAArgs {
     // problem p owns poses [kf_off[p], kf_off[p+1]), points [pt_off[p], ..), observations [obs_off[p], ..)
     const int32_t *kf_off, *pt_off, *obs_off;
-    double* poses;            // g2o order [omega; upsilon], in/out
+    double* poses;            // [t; angle-axis], in/out
     const uint8_t* fixed;
     double* pts;              // in/out
     const int32_t* kf_idx;    // per obs, LOCAL pose index inside the problem
@@ -70,12 +69,11 @@ struct BAArgs {
     double* xl;               // [n_pt][3]
     double* pts_backup;       // [n_pt][3]
     double* scale_l;          // [n_pt][3]  Ceres twin: Jacobi scaling of the landmark columns
-    uint8_t* outlier;         // [n_obs]
-    double* stats;            // [n_problems][8]: iters, trials, chi_first, chi_last, lambda, n_outliers
+    double* stats;            // [n_problems][8]: trials, successful steps, cost_first, cost_last, radius, termination
     float fx, fy, cx, cy;
-    int max_iters, max_trials;
-    double huber_delta, chi2_outlier, tau;
-    const uint8_t* loss_mask;   // Ceres twin: residual blocks that carry the HuberLoss (null = all of them)
+    int max_iters;
+    double huber_delta;
+    const uint8_t* loss_mask;   // residual blocks that carry the HuberLoss (null = all of them)
 };
 
 __device__ __forceinline__ double warp_sum(double v) {
@@ -115,11 +113,6 @@ __device__ double block_max(double v, double* s_tmp) {
     }
     __syncthreads();
     return s_tmp[32];
-}
-
-__device__ __forceinline__ SE3d pose_from_g2o(const double* est) {
-    const double v[6] = {est[3], est[4], est[5], est[0], est[1], est[2]};
-    return se3_exp(v);
 }
 
 __device__ __forceinline__ void inverse3d(const double* H /* row major 3x3 */, double* inv) {
@@ -282,21 +275,18 @@ struct ClusterWs {            // per problem, in global memory
     int ok;
 };
 
-// kCeres = false: ba::LocalBAG2O (g2o Levenberg, Huber kernel, pixel residuals, exp-map pose update)
-// kCeres = true : ba::LocalBA   (Ceres trust-region LM with Jacobi scaling, no loss, normalised residuals, poses as
-//                 [t; angle-axis] with additive updates) -- the same reduction / Schur / Cholesky machinery with
-//                 per-parameter damping d_k = clamp(s_k^2 H_kk, 1e-6, 1e32) / (radius s_k^2) instead of lambda
-template <bool kCeres>
+// ba::LocalBA (Ceres trust-region LM with Jacobi scaling, normalised residuals, optional per-block Huber loss, poses as
+// [t; angle-axis] with additive updates): Schur complement with per-parameter damping
+// d_k = clamp(s_k^2 H_kk, 1e-6, 1e32) / (radius s_k^2)
 __global__ void __launch_bounds__(kBAThreads) local_ba_kernel(const BAArgs a, ClusterWs* __restrict__ ws_all) {
     namespace cg = cooperative_groups;
     cg::cluster_group cluster = cg::this_cluster();
     extern __shared__ double s_mem[];          // CTA 0: S (dimp x dimp) + rhs
     __shared__ double s_tmp[33];
-    __shared__ double s_R[kMaxPoses][12];
-    __shared__ double s_pose[kMaxPoses][6];    // replica of the pose estimates (g2o order)
+    __shared__ double s_pose[kMaxPoses][6];    // replica of the pose estimates [t; angle-axis]
     __shared__ double s_backup[kMaxPoses][6];
     __shared__ double s_xp[kMaxFreePoses * 6];
-    __shared__ double s_sp[kMaxFreePoses * 6];   // Ceres twin: Jacobi scaling of the pose columns
+    __shared__ double s_sp[kMaxFreePoses * 6];   // Jacobi scaling of the pose columns
     __shared__ int s_free[kMaxPoses];
     __shared__ int s_np;
 
@@ -325,12 +315,6 @@ __global__ void __launch_bounds__(kBAThreads) local_ba_kernel(const BAArgs a, Cl
     const int n_pairs = np * (np + 1) / 2;
     int red_slot = 0;
 
-    auto refresh_poses = [&]() {
-        if constexpr (!kCeres) {
-            if (tid < n_kf) se3_to_mat(pose_from_g2o(s_pose[tid]), s_R[tid]);
-        }
-        __syncthreads();
-    };
     // cluster-wide sum of up to 2 values (identical result in every thread of every CTA); contains a cluster barrier
     auto cluster_sum2 = [&](double v0, double v1, double* out0, double* out1) {
         v0 = block_sum(v0, s_tmp);
@@ -353,80 +337,40 @@ __global__ void __launch_bounds__(kBAThreads) local_ba_kernel(const BAArgs a, Cl
     auto reproject = [&](int o, double* e0, double* e1, double* px, double* py, double* pz) {
         const double* X = a.pts + 3 * (size_t)(p0 + a.pt_idx[o0 + o]);
         const double X0 = __ldcg(X), X1 = __ldcg(X + 1), X2 = __ldcg(X + 2);
-        if constexpr (kCeres) {
-            double p[3];
-            ceres_project(s_pose[a.kf_idx[o0 + o]], X0, X1, X2, p);
-            const double iz = 1.0 / p[2];
-            // PinholeCamera::Pixel2Camera2D: float intrinsics, double maths
-            *e0 = (a.obs[2 * (size_t)(o0 + o)] - cx) / fx - p[0] * iz;
-            *e1 = (a.obs[2 * (size_t)(o0 + o) + 1] - cy) / fy - p[1] * iz;
-            *px = p[0]; *py = p[1]; *pz = p[2];
-        } else {
-            const double* Tm = s_R[a.kf_idx[o0 + o]];
-            const double x = Tm[0] * X0 + Tm[1] * X1 + Tm[2] * X2 + Tm[3];
-            const double y = Tm[4] * X0 + Tm[5] * X1 + Tm[6] * X2 + Tm[7];
-            const double z = Tm[8] * X0 + Tm[9] * X1 + Tm[10] * X2 + Tm[11];
-            *e0 = a.obs[2 * (size_t)(o0 + o)] - (x / z * fx + cx);
-            *e1 = a.obs[2 * (size_t)(o0 + o) + 1] - (y / z * fy + cy);
-            *px = x; *py = y; *pz = z;
-        }
+        double p[3];
+        ceres_project(s_pose[a.kf_idx[o0 + o]], X0, X1, X2, p);
+        const double iz = 1.0 / p[2];
+        // PinholeCamera::Pixel2Camera2D: float intrinsics, double maths
+        *e0 = (a.obs[2 * (size_t)(o0 + o)] - cx) / fx - p[0] * iz;
+        *e1 = (a.obs[2 * (size_t)(o0 + o) + 1] - cy) / fy - p[1] * iz;
+        *px = p[0]; *py = p[1]; *pz = p[2];
     };
-    // Ceres twin: LM damping of one parameter from its Hessian diagonal and Jacobi scale
+    // LM damping of one parameter from its Hessian diagonal and Jacobi scale
     double radius = 1e4, decrease_factor = 2.0;
     auto damp = [&](double hkk, double sk) { return fmin(fmax(sk * sk * hkk, 1e-6), 1e32) / radius / (sk * sk); };
-    int term = 0, n_success = 0;   // Ceres twin: termination code (see ygz_b200.h), accepted steps
+    int term = 0, n_success = 0;   // termination code (see ygz_b200.h), accepted steps
 
-    refresh_poses();
-    int iters = 0, trials_total = 0;
-    double chi_first = 0, chi_last = 0, lambda = 0, ni = 2, rho = 0, currentChi = 0;
+    int trials_total = 0;
+    double chi_first = 0, chi_last = 0, rho = 0, currentChi = 0;
 
     for (int iteration = 0; iteration < a.max_iters; ++iteration) {
         // ---- computeActiveErrors + buildSystem -------------------------------------------------------------------
         for (int i = ct; i < np * 36; i += CT) ws.Hpp[i] = 0.0;
         for (int i = ct; i < dimp; i += CT) ws.bp[i] = 0.0;
         double acc = 0;
-        if constexpr (kCeres) {
-            for (int o = ct; o < n_obs; o += CT) {
-                const double* X = a.pts + 3 * (size_t)(p0 + a.pt_idx[o0 + o]);
-                double* rec = a.lin + 21 * (size_t)(o0 + o);
-                ceres_linearise(s_pose[a.kf_idx[o0 + o]], __ldcg(X), __ldcg(X + 1), __ldcg(X + 2),
-                                (a.obs[2 * (size_t)(o0 + o)] - cx) / fx, (a.obs[2 * (size_t)(o0 + o) + 1] - cy) / fy, rec);
-                // ceres::HuberLoss through the Corrector: rho'' <= 0, so the block is weighted by rho' = a / |r| beyond a
-                const double e2 = rec[0] * rec[0] + rec[1] * rec[1];
-                if (a.huber_delta > 0 && e2 > dsqr && (!a.loss_mask || a.loss_mask[o0 + o])) {
-                    const double rt = sqrt(e2);
-                    rec[2] = a.huber_delta / rt;
-                    acc += 2 * a.huber_delta * rt - dsqr;
-                } else {
-                    acc += e2;
-                }
-            }
-        } else {
-            for (int o = ct; o < n_obs; o += CT) {
-                double e0, e1, x, y, z;
-                reproject(o, &e0, &e1, &x, &y, &z);
-                const double e2 = e0 * e0 + e1 * e1;
-                double w = 1.0;
-                if (a.huber_delta > 0 && e2 > dsqr) {
-                    w = a.huber_delta / sqrt(e2);
-                    acc += 2 * sqrt(e2) * a.huber_delta - dsqr;
-                } else {
-                    acc += e2;
-                }
-                const double* Tm = s_R[a.kf_idx[o0 + o]];
-                double* rec = a.lin + 21 * (size_t)(o0 + o);
-                rec[0] = e0; rec[1] = e1; rec[2] = w;
-                const double z_2 = z * z, iz = -1. / z;
-                const double t02 = -x / z * fx, t12 = -y / z * fy;
-#pragma unroll
-                for (int c = 0; c < 3; ++c) {
-                    rec[3 + c] = iz * (fx * Tm[c] + t02 * Tm[8 + c]);
-                    rec[6 + c] = iz * (fy * Tm[4 + c] + t12 * Tm[8 + c]);
-                }
-                rec[9] = x * y / z_2 * fx; rec[10] = -(1 + (x * x / z_2)) * fx; rec[11] = y / z * fx;
-                rec[12] = -1. / z * fx; rec[13] = 0; rec[14] = x / z_2 * fx;
-                rec[15] = (1 + y * y / z_2) * fy; rec[16] = -x * y / z_2 * fy; rec[17] = -x / z * fy;
-                rec[18] = 0; rec[19] = -1. / z * fy; rec[20] = y / z_2 * fy;
+        for (int o = ct; o < n_obs; o += CT) {
+            const double* X = a.pts + 3 * (size_t)(p0 + a.pt_idx[o0 + o]);
+            double* rec = a.lin + 21 * (size_t)(o0 + o);
+            ceres_linearise(s_pose[a.kf_idx[o0 + o]], __ldcg(X), __ldcg(X + 1), __ldcg(X + 2),
+                            (a.obs[2 * (size_t)(o0 + o)] - cx) / fx, (a.obs[2 * (size_t)(o0 + o) + 1] - cy) / fy, rec);
+            // ceres::HuberLoss through the Corrector: rho'' <= 0, so the block is weighted by rho' = a / |r| beyond a
+            const double e2 = rec[0] * rec[0] + rec[1] * rec[1];
+            if (a.huber_delta > 0 && e2 > dsqr && (!a.loss_mask || a.loss_mask[o0 + o])) {
+                const double rt = sqrt(e2);
+                rec[2] = a.huber_delta / rt;
+                acc += 2 * a.huber_delta * rt - dsqr;
+            } else {
+                acc += e2;
             }
         }
         double dummy;
@@ -451,14 +395,10 @@ __global__ void __launch_bounds__(kBAThreads) local_ba_kernel(const BAArgs a, Cl
             Hj[0] = H[0]; Hj[1] = H[1]; Hj[2] = H[2]; Hj[3] = H[1]; Hj[4] = H[3]; Hj[5] = H[4]; Hj[6] = H[2]; Hj[7] = H[4]; Hj[8] = H[5];
             double* bj = a.bl + 3 * (size_t)(p0 + j);
             bj[0] = b[0]; bj[1] = b[1]; bj[2] = b[2];
-            if constexpr (kCeres) {
-                mx = fmax(mx, fmax(fabs(b[0]), fmax(fabs(b[1]), fabs(b[2]))));   // gradient max norm
-                if (iteration == 0) {  // Jacobi scaling from the initial Jacobian: 1 / (1 + ||column||)
-                    double* sj = a.scale_l + 3 * (size_t)(p0 + j);
-                    sj[0] = 1.0 / (1.0 + sqrt(H[0])); sj[1] = 1.0 / (1.0 + sqrt(H[3])); sj[2] = 1.0 / (1.0 + sqrt(H[5]));
-                }
-            } else {
-                mx = fmax(mx, fmax(fabs(H[0]), fmax(fabs(H[3]), fabs(H[5]))));
+            mx = fmax(mx, fmax(fabs(b[0]), fmax(fabs(b[1]), fabs(b[2]))));   // gradient max norm
+            if (iteration == 0) {  // Jacobi scaling from the initial Jacobian: 1 / (1 + ||column||)
+                double* sj = a.scale_l + 3 * (size_t)(p0 + j);
+                sj[0] = 1.0 / (1.0 + sqrt(H[0])); sj[1] = 1.0 / (1.0 + sqrt(H[3])); sj[2] = 1.0 / (1.0 + sqrt(H[5]));
             }
         }
         // Hpp, bp : (free pose, chunk) tasks over all warps of the cluster, f64 atomics into the workspace
@@ -503,32 +443,23 @@ __global__ void __launch_bounds__(kBAThreads) local_ba_kernel(const BAArgs a, Cl
             }
         }
         {
-            double m0, m1;
-            // max |diag| via two sums is wrong; use a dedicated max reduction through the same partial slots
+            // gradient max norm: a max reduction through the partial slots of cluster_sum2
             const double bm = block_max(mx, s_tmp);
             const int slot = red_slot;
             red_slot = (red_slot + 1) & 3;
             if (tid == 0) ws.red[slot][rank][0] = bm;
             cluster.sync();                                   // also publishes Hll/bl and the Hpp/bp atomics
-            m0 = 0;
+            double m0 = 0;
             for (int r = 0; r < C; ++r) m0 = fmax(m0, __ldcg(&ws.red[slot][r][0]));
-            if constexpr (kCeres) {
-                for (int i = 0; i < dimp; ++i) m0 = fmax(m0, fabs(__ldcg(&ws.bp[i])));
-                if (iteration == 0) {
-                    if (tid < dimp) s_sp[tid] = 1.0 / (1.0 + sqrt(__ldcg(&ws.Hpp[(tid / 6) * 36 + (tid % 6) * 7])));
-                    __syncthreads();
-                }
-                if (m0 <= 1e-10) term = 1;   // gradient tolerance
-            } else if (iteration == 0) {  // computeLambdaInit = tau * max |diag H|
-                for (int i = 0; i < dimp; ++i) m0 = fmax(m0, fabs(__ldcg(&ws.Hpp[(i / 6) * 36 + (i % 6) * 7])));
-                lambda = a.tau * m0;
-                ni = 2;
+            for (int i = 0; i < dimp; ++i) m0 = fmax(m0, fabs(__ldcg(&ws.bp[i])));
+            if (iteration == 0) {
+                if (tid < dimp) s_sp[tid] = 1.0 / (1.0 + sqrt(__ldcg(&ws.Hpp[(tid / 6) * 36 + (tid % 6) * 7])));
+                __syncthreads();
             }
-            (void)m1;
+            if (m0 <= 1e-10) term = 1;   // gradient tolerance
         }
-        if (kCeres && term) break;
+        if (term) break;
 
-        int qmax = 0;
         do {
             // _optimizer->push(): pose replica in shared memory, landmarks per owner thread
             if (tid < n_kf)
@@ -538,12 +469,8 @@ __global__ void __launch_bounds__(kBAThreads) local_ba_kernel(const BAArgs a, Cl
                 const double* Hj = a.Hll + 9 * (size_t)(p0 + j);
 #pragma unroll
                 for (int t = 0; t < 9; ++t) D[t] = Hj[t];
-                if constexpr (kCeres) {
-                    const double* sj = a.scale_l + 3 * (size_t)(p0 + j);
-                    D[0] += damp(Hj[0], sj[0]); D[4] += damp(Hj[4], sj[1]); D[8] += damp(Hj[8], sj[2]);
-                } else {
-                    D[0] += lambda; D[4] += lambda; D[8] += lambda;
-                }
+                const double* sj = a.scale_l + 3 * (size_t)(p0 + j);
+                D[0] += damp(Hj[0], sj[0]); D[4] += damp(Hj[4], sj[1]); D[8] += damp(Hj[8], sj[2]);
                 inverse3d(D, a.Dinv + 9 * (size_t)(p0 + j));
 #pragma unroll
                 for (int c = 0; c < 3; ++c) a.pts_backup[3 * (size_t)(p0 + j) + c] = a.pts[3 * (size_t)(p0 + j) + c];
@@ -613,14 +540,14 @@ __global__ void __launch_bounds__(kBAThreads) local_ba_kernel(const BAArgs a, Cl
                 }
             }
             cluster.sync();
-            // CTA 0: S = Hpp + lambda I - sum, dense Cholesky in shared memory, triangular solves by warp 0
+            // CTA 0: S = Hpp + D - sum, dense Cholesky in shared memory, triangular solves by warp 0
             if (rank == 0) {
                 for (int i = tid; i < dimp * dimp; i += T) {
                     const int r = i / dimp, c = i - r * dimp;
                     double v = __ldcg(&ws.S[i]);
                     if (r / 6 == c / 6) {
                         const double h = __ldcg(&ws.Hpp[(r / 6) * 36 + (r % 6) * 6 + (c % 6)]);
-                        v += h + (r == c ? (kCeres ? damp(h, s_sp[r]) : lambda) : 0.0);
+                        v += h + (r == c ? damp(h, s_sp[r]) : 0.0);
                     }
                     s_S[i] = v;
                 }
@@ -694,135 +621,84 @@ __global__ void __launch_bounds__(kBAThreads) local_ba_kernel(const BAArgs a, Cl
 #pragma unroll
                 for (int c = 0; c < 3; ++c) {
                     const double x = Di[3 * c] * r[0] + Di[3 * c + 1] * r[1] + Di[3 * c + 2] * r[2];
-                    if constexpr (kCeres) {
-                        a.xl[3 * (size_t)(p0 + j) + c] = x;   // the model cost change needs J delta per observation
-                        scale += x * x;                      // |step|^2
-                        xnorm2 += X[c] * X[c];
-                    } else {
-                        scale += x * (lambda * x + bj[c]);
-                    }
+                    a.xl[3 * (size_t)(p0 + j) + c] = x;   // the model cost change needs J delta per observation
+                    scale += x * x;                      // |step|^2
+                    xnorm2 += X[c] * X[c];
                     X[c] += x;
                 }
             }
-            if constexpr (kCeres) {
-                if (rank == 0 && tid < n_kf && s_free[tid] >= 0) {
-                    const double* u = s_xp + 6 * s_free[tid];
+            if (rank == 0 && tid < n_kf && s_free[tid] >= 0) {
+                const double* u = s_xp + 6 * s_free[tid];
 #pragma unroll
-                    for (int c = 0; c < 6; ++c) {
-                        scale += u[c] * u[c];
-                        xnorm2 += s_pose[tid][c] * s_pose[tid][c];
-                    }
+                for (int c = 0; c < 6; ++c) {
+                    scale += u[c] * u[c];
+                    xnorm2 += s_pose[tid][c] * s_pose[tid][c];
                 }
-                if (tid < n_kf && s_free[tid] >= 0) {  // plain Euclidean parameter block: x + delta
-                    const double* u = s_xp + 6 * s_free[tid];
+            }
+            if (tid < n_kf && s_free[tid] >= 0) {  // plain Euclidean parameter block: x + delta
+                const double* u = s_xp + 6 * s_free[tid];
 #pragma unroll
-                    for (int c = 0; c < 6; ++c) s_pose[tid][c] += u[c];
-                }
-            } else {
-                if (rank == 0 && tid < dimp) scale += s_xp[tid] * (lambda * s_xp[tid] + __ldcg(&ws.bp[tid]));
-                if (tid < n_kf && s_free[tid] >= 0) {  // VertexSE3Sophus::oplusImpl on the replica
-                    const double* u = s_xp + 6 * s_free[tid];
-                    const double v[6] = {u[3], u[4], u[5], u[0], u[1], u[2]};
-                    const SE3d Tn = se3_mul(se3_exp(v), pose_from_g2o(s_pose[tid]));
-                    double lg[6];
-                    se3_log(Tn, lg);
-                    s_pose[tid][0] = lg[3]; s_pose[tid][1] = lg[4]; s_pose[tid][2] = lg[5];
-                    s_pose[tid][3] = lg[0]; s_pose[tid][4] = lg[1]; s_pose[tid][5] = lg[2];
-                }
+                for (int c = 0; c < 6; ++c) s_pose[tid][c] += u[c];
             }
             __syncthreads();
-            refresh_poses();
-            double scale_tot, dummy2;
-            bool accept;
-            if constexpr (kCeres) {
-                double step2, x2;
-                cluster_sum2(scale, xnorm2, &step2, &x2);   // (barrier: updated landmarks and xl visible cluster-wide)
-                // candidate cost and model cost change -(J delta)^T (r + J delta / 2), one pass over the observations
-                double newc = 0, model = 0;
-                for (int o = ct; o < n_obs; o += CT) {
-                    double e0, e1, x, y, z;
-                    reproject(o, &e0, &e1, &x, &y, &z);
-                    const double e2n = e0 * e0 + e1 * e1;
-                    newc += (a.huber_delta > 0 && e2n > dsqr && (!a.loss_mask || a.loss_mask[o0 + o])) ? 2 * a.huber_delta * sqrt(e2n) - dsqr : e2n;
-                    const double* rec = a.lin + 21 * (size_t)(o0 + o);
-                    const int fi = s_free[a.kf_idx[o0 + o]];
-                    const double* dl = a.xl + 3 * (size_t)(p0 + a.pt_idx[o0 + o]);
-                    const double d0 = __ldcg(dl), d1 = __ldcg(dl + 1), d2 = __ldcg(dl + 2);
+            double step2, x2;
+            cluster_sum2(scale, xnorm2, &step2, &x2);   // (barrier: updated landmarks and xl visible cluster-wide)
+            // candidate cost and model cost change -(J delta)^T (r + J delta / 2), one pass over the observations
+            double newc = 0, model = 0;
+            for (int o = ct; o < n_obs; o += CT) {
+                double e0, e1, x, y, z;
+                reproject(o, &e0, &e1, &x, &y, &z);
+                const double e2n = e0 * e0 + e1 * e1;
+                newc += (a.huber_delta > 0 && e2n > dsqr && (!a.loss_mask || a.loss_mask[o0 + o])) ? 2 * a.huber_delta * sqrt(e2n) - dsqr : e2n;
+                const double* rec = a.lin + 21 * (size_t)(o0 + o);
+                const int fi = s_free[a.kf_idx[o0 + o]];
+                const double* dl = a.xl + 3 * (size_t)(p0 + a.pt_idx[o0 + o]);
+                const double d0 = __ldcg(dl), d1 = __ldcg(dl + 1), d2 = __ldcg(dl + 2);
 #pragma unroll
-                    for (int row = 0; row < 2; ++row) {
-                        double jy = 0;
-                        if (fi >= 0) {
+                for (int row = 0; row < 2; ++row) {
+                    double jy = 0;
+                    if (fi >= 0) {
 #pragma unroll
-                            for (int k = 0; k < 6; ++k) jy += rec[9 + 6 * row + k] * s_xp[6 * fi + k];
-                        }
-                        jy += rec[3 + 3 * row] * d0;
-                        jy += rec[4 + 3 * row] * d1;
-                        jy += rec[5 + 3 * row] * d2;
-                        model -= rec[2] * jy * (rec[row] + jy / 2);
+                        for (int k = 0; k < 6; ++k) jy += rec[9 + 6 * row + k] * s_xp[6 * fi + k];
                     }
-                }
-                double newc_tot, model_tot;
-                cluster_sum2(newc, model, &newc_tot, &model_tot);
-                const double cost = 0.5 * currentChi, new_cost = 0.5 * newc_tot;
-                bool accepted = false;
-                double relative_decrease = 0;
-                if (ok2 && model_tot > 0) {
-                    relative_decrease = (cost - new_cost) / model_tot;
-                    accepted = relative_decrease > 1e-3;
-                }
-                accept = accepted;
-                if (accepted) {
-                    if (sqrt(step2) <= 1e-8 * (sqrt(x2) + 1e-8)) {  // parameter tolerance: checked before the step is taken
-                        term = 2;
-                        accept = false;
-                    } else {
-                        ++n_success;
-                        currentChi = newc_tot;
-                        if (fabs(cost - new_cost) <= 1e-6 * cost) {
-                            term = 3;   // function tolerance
-                        } else {
-                            {
-                            const double t3 = 2.0 * relative_decrease - 1.0;
-                            radius = radius / fmax(1.0 / 3.0, 1.0 - t3 * t3 * t3);
-                        }
-                            radius = fmin(1e16, radius);
-                            decrease_factor = 2.0;
-                        }
-                    }
-                } else {
-                    radius = radius / decrease_factor;
-                    decrease_factor *= 2.0;
-                    if (radius < 1e-32) term = 4;
-                }
-                rho = accepted ? 1.0 : -1.0;
-                (void)scale_tot; (void)dummy2;
-            } else {
-                cluster_sum2(scale, 0.0, &scale_tot, &dummy2);    // (barrier: updated landmarks visible cluster-wide)
-                scale_tot += 1e-3;
-                double chi_part = 0;
-                for (int o = ct; o < n_obs; o += CT) {
-                    double e0, e1, x, y, z;
-                    reproject(o, &e0, &e1, &x, &y, &z);
-                    const double e2 = e0 * e0 + e1 * e1;
-                    chi_part += (a.huber_delta > 0 && e2 > dsqr) ? 2 * sqrt(e2) * a.huber_delta - dsqr : e2;
-                }
-                double tempChi;
-                cluster_sum2(chi_part, 0.0, &tempChi, &dummy2);
-                if (!ok2) tempChi = 1.7976931348623157e308;
-                rho = (currentChi - tempChi) / scale_tot;
-                if (rho > 0 && isfinite(tempChi)) {
-                    double alpha = 1. - pow((2 * rho - 1), 3);
-                    alpha = fmin(alpha, 2. / 3.);
-                    lambda *= fmax(1. / 3., alpha);
-                    ni = 2;
-                    currentChi = tempChi;
-                    accept = true;
-                } else {
-                    lambda *= ni;
-                    ni *= 2;
-                    accept = false;
+                    jy += rec[3 + 3 * row] * d0;
+                    jy += rec[4 + 3 * row] * d1;
+                    jy += rec[5 + 3 * row] * d2;
+                    model -= rec[2] * jy * (rec[row] + jy / 2);
                 }
             }
+            double newc_tot, model_tot;
+            cluster_sum2(newc, model, &newc_tot, &model_tot);
+            const double cost = 0.5 * currentChi, new_cost = 0.5 * newc_tot;
+            bool accepted = false;
+            double relative_decrease = 0;
+            if (ok2 && model_tot > 0) {
+                relative_decrease = (cost - new_cost) / model_tot;
+                accepted = relative_decrease > 1e-3;
+            }
+            bool accept = accepted;
+            if (accepted) {
+                if (sqrt(step2) <= 1e-8 * (sqrt(x2) + 1e-8)) {  // parameter tolerance: checked before the step is taken
+                    term = 2;
+                    accept = false;
+                } else {
+                    ++n_success;
+                    currentChi = newc_tot;
+                    if (fabs(cost - new_cost) <= 1e-6 * cost) {
+                        term = 3;   // function tolerance
+                    } else {
+                        const double t3 = 2.0 * relative_decrease - 1.0;
+                        radius = radius / fmax(1.0 / 3.0, 1.0 - t3 * t3 * t3);
+                        radius = fmin(1e16, radius);
+                        decrease_factor = 2.0;
+                    }
+                }
+            } else {
+                radius = radius / decrease_factor;
+                decrease_factor *= 2.0;
+                if (radius < 1e-32) term = 4;
+            }
+            rho = accepted ? 1.0 : -1.0;
             if (!accept) {  // _optimizer->pop()
                 if (tid < n_kf)
                     for (int c = 0; c < 6; ++c) s_pose[tid][c] = s_backup[tid][c];
@@ -830,42 +706,19 @@ __global__ void __launch_bounds__(kBAThreads) local_ba_kernel(const BAArgs a, Cl
 #pragma unroll
                     for (int c = 0; c < 3; ++c) a.pts[3 * (size_t)(p0 + j) + c] = a.pts_backup[3 * (size_t)(p0 + j) + c];
                 __syncthreads();
-                refresh_poses();
             }
-            ++qmax;
             ++trials_total;
-        } while (kCeres ? (rho < 0 && !term && trials_total < a.max_iters) : (rho < 0 && qmax < a.max_trials));
-        ++iters;
+        } while (rho < 0 && !term && trials_total < a.max_iters);
         chi_last = currentChi;
-        if constexpr (kCeres) {
-            if (term || trials_total >= a.max_iters) break;
-        } else {
-            if (qmax == a.max_trials || rho == 0) break;
-        }
+        if (term || trials_total >= a.max_iters) break;
     }
-    cluster.sync();  // a rejected last trial restored landmarks owned by other CTAs
-    // outlier flags (BA.cpp:505-515): plain chi2 > 5.991
-    double n_out = 0;
-    for (int o = ct; o < n_obs; o += CT) {
-        double e0, e1, x, y, z;
-        reproject(o, &e0, &e1, &x, &y, &z);
-        const int out = (!kCeres && e0 * e0 + e1 * e1 > a.chi2_outlier) ? 1 : 0;   // ba::LocalBA marks nothing
-        a.outlier[o0 + o] = (uint8_t)out;
-        n_out += out;
-    }
-    double n_out_tot, dummy3;
-    cluster_sum2(n_out, 0.0, &n_out_tot, &dummy3);
     if (rank == 0) {
         if (tid < n_kf)
             for (int c = 0; c < 6; ++c) a.poses[6 * (size_t)(k0 + tid) + c] = s_pose[tid][c];
         if (tid == 0) {
             double* st = a.stats + 8 * (size_t)prob;
-            if constexpr (kCeres) {
-                st[0] = trials_total; st[1] = n_success; st[2] = 0.5 * chi_first; st[3] = 0.5 * chi_last; st[4] = radius; st[5] = term;
-            } else {
-                st[0] = iters; st[1] = trials_total; st[2] = chi_first; st[3] = chi_last; st[4] = lambda; st[5] = n_out_tot;
-            }
-            st[6] = 0.0; st[7] = 0.0;   // (unused by this kernel generation; the host copies all 8 slots)
+            st[0] = trials_total; st[1] = n_success; st[2] = 0.5 * chi_first; st[3] = 0.5 * chi_last; st[4] = radius; st[5] = term;
+            st[6] = 0.0; st[7] = 0.0;   // (unused by this kernel; the host copies all 8 slots)
         }
     }
 }
@@ -1456,19 +1309,17 @@ int run_local_ba2(ygzb_ctx* ctx, int n_problems, const int32_t* kf_off, const in
     return YGZB_OK;
 }
 
-// shared body of ygzb_local_ba (ceres = false) and ygzb_local_ba_ceres (ceres = true): index bookkeeping on the host,
-// one cluster launch, results back.  hst receives the 8 raw statistics of every problem.
-int run_local_ba(ygzb_ctx* ctx, bool ceres, int n_problems, const int32_t* kf_off, const int32_t* pt_off, const int32_t* obs_off,
+// shared body of ygzb_local_ba_ceres and ygzb_two_view_ba: index bookkeeping on the host, one cluster launch, results
+// back.  hst receives the 8 raw statistics of every problem.
+int run_local_ba(ygzb_ctx* ctx, int n_problems, const int32_t* kf_off, const int32_t* pt_off, const int32_t* obs_off,
                  double* poses, const uint8_t* fixed, double* pts, const int32_t* kf_idx, const int32_t* pt_idx,
-                 const double* obs_px, const ygzb_ba_params* prm, uint8_t* outlier, std::vector<double>& hst,
-                 const uint8_t* loss_mask = nullptr) {
+                 const double* obs_px, const ygzb_ba_params* prm, std::vector<double>& hst, const uint8_t* loss_mask = nullptr) {
     cudaSetDevice(ctx->device);
     for (const auto& oc : {std::make_pair(kf_off, "kf_off"), std::make_pair(pt_off, "pt_off"), std::make_pair(obs_off, "obs_off")}) {
         const int rc = check_offsets(ctx, oc.first, n_problems, oc.second);
         if (rc != YGZB_OK) return rc;
     }
     const size_t P = (size_t)n_problems, NK = (size_t)kf_off[n_problems], NP = (size_t)pt_off[n_problems], NO = (size_t)obs_off[n_problems];
-    if (!ceres && !getenv("YGZB_BA_GEN1")) return run_local_ba2(ctx, n_problems, kf_off, pt_off, obs_off, poses, fixed, pts, kf_idx, pt_idx, obs_px, prm, outlier, hst);
     // ---- structure: observations grouped by landmark, by pose, and landmark-sharing observation pairs per block pair
     std::vector<int32_t> lm_start(NP + 1, 0), lm_obs(NO), ps_start(NK + 1, 0), ps_obs(NO), pair_off(P + 1, 0), pair_start, pair_o1, pair_o2;
     int max_free = 0;
@@ -1554,7 +1405,7 @@ int run_local_ba(ygzb_ctx* ctx, bool ceres, int n_problems, const int32_t* kf_of
     sz.take<int32_t>(3 * (P + 1)); sz.take<double>(6 * NK); sz.take<uint8_t>(NK); sz.take<double>(3 * NP); sz.take<int32_t>(2 * NO);
     sz.take<double>(2 * NO); sz.take<int32_t>(NP + 1 + NO + NK + 1 + NO); sz.take<int32_t>(P + 1 + NPS + 2 * NPAIR);
     sz.take<double>(21 * NO); sz.take<double>(9 * NP); sz.take<double>(3 * NP); sz.take<double>(9 * NP); sz.take<double>(3 * NP);
-    sz.take<double>(3 * NP); sz.take<double>(3 * NP); sz.take<uint8_t>(NO); sz.take<double>(8 * P);
+    sz.take<double>(3 * NP); sz.take<double>(3 * NP); sz.take<double>(8 * P);
     void* buf = dev_scratch(ctx, 7, sz.bytes());
     if (!buf) return YGZB_ERR_CUDA;
     Carver c(buf);
@@ -1574,7 +1425,6 @@ int run_local_ba(ygzb_ctx* ctx, bool ceres, int n_problems, const int32_t* kf_of
     a.xl = c.take<double>(3 * NP);
     a.pts_backup = c.take<double>(3 * NP);
     a.scale_l = c.take<double>(3 * NP);
-    a.outlier = c.take<uint8_t>(NO);
     a.stats = c.take<double>(8 * P);
     // kf_idx / pt_idx stay LOCAL to the problem; lm_obs / ps_obs / pair entries are GLOBAL observation ids.
     // All inputs sit at the front of the device buffer in one contiguous run: they are assembled in a pinned staging
@@ -1609,8 +1459,7 @@ int run_local_ba(ygzb_ctx* ctx, bool ceres, int n_problems, const int32_t* kf_of
     a.lm_start = d_csr; a.lm_obs = d_csr + NP + 1; a.ps_start = d_csr + NP + 1 + NO; a.ps_obs = d_csr + NP + 1 + NO + NK + 1;
     a.pair_off = d_pairs; a.pair_start = d_pairs + P + 1; a.pair_o1 = d_pairs + P + 1 + NPS; a.pair_o2 = d_pairs + P + 1 + NPS + NPAIR;
     a.fx = ctx->prm.fx; a.fy = ctx->prm.fy; a.cx = ctx->prm.cx; a.cy = ctx->prm.cy;
-    a.max_iters = prm->max_iters; a.max_trials = prm->max_trials; a.huber_delta = prm->huber_delta;
-    a.chi2_outlier = prm->chi2_outlier; a.tau = prm->tau;
+    a.max_iters = prm->max_iters; a.huber_delta = prm->huber_delta;
     a.loss_mask = nullptr;
     if (loss_mask && NO) {
         uint8_t* d_mask = static_cast<uint8_t*>(dev_scratch(ctx, 4, NO));
@@ -1622,15 +1471,13 @@ int run_local_ba(ygzb_ctx* ctx, bool ceres, int n_problems, const int32_t* kf_of
     const size_t smem = sizeof(double) * ((size_t)dimp * dimp + (size_t)dimp);
     ClusterWs* d_ws = static_cast<ClusterWs*>(dev_scratch(ctx, 5, sizeof(ClusterWs) * P));
     if (!d_ws) return YGZB_ERR_CUDA;
-    auto kernel = ceres ? local_ba_kernel<true> : local_ba_kernel<false>;
     {
-        // opt both instantiations in to the largest reduced system (16 free poses: 74.5 KB) once: a per-call value would race
-        // between the contexts of several host threads
+        // opt in to the largest reduced system (16 free poses: 74.5 KB) once: a per-call value would race between the
+        // contexts of several host threads
         static std::once_flag smem_once;
         std::call_once(smem_once, [] {
             const int max_smem = (int)(sizeof(double) * ((size_t)(6 * kMaxFreePoses) * (6 * kMaxFreePoses) + 6 * kMaxFreePoses));
-            cudaFuncSetAttribute(local_ba_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
-            cudaFuncSetAttribute(local_ba_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
+            cudaFuncSetAttribute(local_ba_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
         });
     }
     {
@@ -1644,7 +1491,7 @@ int run_local_ba(ygzb_ctx* ctx, bool ceres, int n_problems, const int32_t* kf_of
             const int v = atoi(e);
             if (v == 1 || v == 2 || v == 4 || v == 8 || v == 16) cluster = v;
         }
-        if (cluster > 8) YGZB_CUDA(ctx, cudaFuncSetAttribute(kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
+        if (cluster > 8) YGZB_CUDA(ctx, cudaFuncSetAttribute(local_ba_kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
         cudaLaunchConfig_t cfg{};
         cfg.gridDim = dim3((unsigned)(n_problems * cluster));
         cfg.blockDim = dim3(kBAThreads);
@@ -1658,12 +1505,11 @@ int run_local_ba(ygzb_ctx* ctx, bool ceres, int n_problems, const int32_t* kf_of
         cfg.attrs = attr;
         cfg.numAttrs = 1;
         ProfScope ps(ctx, kStageLocalBA);
-        YGZB_CUDA(ctx, cudaLaunchKernelEx(&cfg, kernel, a, d_ws));
+        YGZB_CUDA(ctx, cudaLaunchKernelEx(&cfg, local_ba_kernel, a, d_ws));
     }
     YGZB_LAUNCHED(ctx);
     TRY(d2h(ctx, poses, d_poses, 6 * NK));
     TRY(d2h(ctx, pts, d_pts, 3 * NP));
-    if (outlier) TRY(d2h(ctx, outlier, a.outlier, NO));
     hst.resize(8 * P);
     TRY(d2h(ctx, hst.data(), a.stats, 8 * P));
     YGZB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
@@ -1679,9 +1525,14 @@ int ygzb_local_ba(ygzb_ctx* ctx, int n_problems, const int32_t* kf_off, const in
     if (!ctx || n_problems < 1 || !kf_off || !pt_off || !obs_off || !poses || !fixed || !pts || !kf_idx || !pt_idx || !obs_px ||
         !prm || !outlier)
         return YGZB_ERR_INVALID;
+    cudaSetDevice(ctx->device);
+    for (const auto& oc : {std::make_pair(kf_off, "kf_off"), std::make_pair(pt_off, "pt_off"), std::make_pair(obs_off, "obs_off")}) {
+        const int rc = check_offsets(ctx, oc.first, n_problems, oc.second);
+        if (rc != YGZB_OK) return rc;
+    }
     std::vector<double> hst;
     try {   // the header promises that calls never throw: allocation failures of the host-side bookkeeping become an error code
-        TRY(run_local_ba(ctx, false, n_problems, kf_off, pt_off, obs_off, poses, fixed, pts, kf_idx, pt_idx, obs_px, prm, outlier, hst));
+        TRY(run_local_ba2(ctx, n_problems, kf_off, pt_off, obs_off, poses, fixed, pts, kf_idx, pt_idx, obs_px, prm, outlier, hst));
     } catch (const std::exception& e) {
         return set_error(ctx, YGZB_ERR_INVALID, "ygzb_local_ba: %s", e.what());
     }
@@ -1709,7 +1560,7 @@ int ygzb_local_ba_ceres(ygzb_ctx* ctx, int n_problems, const int32_t* kf_off, co
     prm.huber_delta = huber_a;   // 0: no loss function (nullptr in AddResidualBlock, BA.cpp:346,364); 0.1: BA.cpp:108-135
     std::vector<double> hst;
     try {
-        TRY(run_local_ba(ctx, true, n_problems, kf_off, pt_off, obs_off, poses, fixed, pts, kf_idx, pt_idx, obs_px, &prm, nullptr, hst));
+        TRY(run_local_ba(ctx, n_problems, kf_off, pt_off, obs_off, poses, fixed, pts, kf_idx, pt_idx, obs_px, &prm, hst));
     } catch (const std::exception& e) {
         return set_error(ctx, YGZB_ERR_INVALID, "ygzb_local_ba_ceres: %s", e.what());
     }
@@ -1802,8 +1653,8 @@ int ygzb_two_view_ba(ygzb_ctx* ctx, int n_problems, const int32_t* offsets, cons
         prm.max_iters = 50;
         prm.huber_delta = 0.1;
         std::vector<double> hst;
-        TRY(run_local_ba(ctx, true, n_problems, kf_off.data(), pt_off.data(), obs_off.data(), poses.data(), fixed.data(), X.data(),
-                         kf_idx.data(), pt_idx.data(), obs.data(), &prm, nullptr, hst, mask.data()));
+        TRY(run_local_ba(ctx, n_problems, kf_off.data(), pt_off.data(), obs_off.data(), poses.data(), fixed.data(), X.data(),
+                         kf_idx.data(), pt_idx.data(), obs.data(), &prm, hst, mask.data()));
         if (stats)
             for (size_t p = 0; p < P; ++p) {
                 stats[p].iters = (int)hst[8 * p]; stats[p].successful_steps = (int)hst[8 * p + 1]; stats[p].cost_initial = hst[8 * p + 2];

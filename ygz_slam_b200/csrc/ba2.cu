@@ -1,6 +1,6 @@
 // ba2.cu -- ba::LocalBAG2O, second generation: a landmark-partitioned thread-block cluster per problem.
 //
-// Replaces (same maths as the first-generation kernel in ba.cu, which stays in service for the Ceres twin):
+// Replaces:
 //   ba::LocalBAG2O                   reference src/Algorithm/BA.cpp:386-543
 //   VertexSE3Sophus::oplusImpl       reference include/ygz/G2oTypes.h:38-45
 //   EdgeSophusSE3ProjectXYZ          reference include/ygz/G2oTypes.h:84-132 (computeError, linearizeOplus)

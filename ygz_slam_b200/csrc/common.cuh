@@ -166,12 +166,12 @@ int launch_align1d(ygzb_frames* f, int n, const int32_t* d_slot, const uint8_t* 
 int launch_project_align(ygzb_frames* f, int n, const int32_t* d_ref_slot, const int32_t* d_cur_slot, const double* d_poses,
                          const int32_t* d_ref_pose, const int32_t* d_cur_pose, const double* d_ref_px, const double* d_ref_depth,
                          const uint8_t* d_ref_level, double* d_cur_px, uint8_t* d_search_level, uint8_t* d_ok);
+// max_feat: the largest feature count of a problem; d_feat_scratch: sparse_align_scratch_bytes(d_offsets[n_problems])
 int launch_sparse_align(ygzb_frames* f, int n_problems, const int32_t* d_ref_slot, const int32_t* d_cur_slot,
-                        const int32_t* d_offsets, const double* d_px, const double* d_depth, const uint8_t* d_has_mp,
+                        const int32_t* d_offsets, int max_feat, const double* d_px, const double* d_depth, const uint8_t* d_has_mp,
                         const double* d_T_ref, double* d_T_cur, int max_level, int min_level, int n_iter, double eps,
-                        int32_t* d_n_meas, int32_t* d_iters, float* d_ref_patch, float* d_gdx, float* d_gdy, double* d_frame_jac,
-                        uint8_t* d_visible, double* d_ws);
-size_t sparse_align_ws_doubles(int n_problems);   // size of d_ws
+                        int32_t* d_n_meas, int32_t* d_iters, void* d_feat_scratch);
+size_t sparse_align_scratch_bytes(size_t n_features);
 
 // bump allocator over one scratch buffer (all sub-buffers 256-byte aligned)
 struct Carver {

@@ -404,10 +404,7 @@ int ygzb_tracker_create(ygzb_frames* f, int n_streams, int max_jobs, const doubl
             b.ref_slot = c.take<int32_t>(J); b.cur_slot = c.take<int32_t>(J); b.offsets = c.take<int32_t>(J + 1); b.in_off = c.take<int32_t>(J);
             b.n_feat = c.take<int32_t>(J); b.n_meas = c.take<int32_t>(J);
             b.T_ref = c.take<double>(J * 12); b.T_cur = c.take<double>(J * 12);
-            b.ref_patch = c.take<float>(F * 16); b.gdx = c.take<float>(F * 16); b.gdy = c.take<float>(F * 16);
-            b.frame_jac = c.take<double>(F * 12); b.visible = c.take<uint8_t>(F);
-            b.sparse_ws = c.take<double>(sparse_align_ws_doubles((int)J));
-            b.sa2_scratch = c.take<double>(sparse_align2_scratch_bytes((int)J, (int)cells) / 8 + 1);
+            b.feat_scratch = c.take<uint8_t>(sparse_align_scratch_bytes(F));
             b.aligned = c.take<int32_t>(J); b.rel = c.take<double>(J * kTrackMaxLocal * 12);
             b.cand_ok = c.take<uint8_t>(Cn); b.cand_px = c.take<double>(Cn * 2); b.n_cand = c.take<int32_t>(J);
             b.c_cnt = c.take<int32_t>(J); b.c_off = c.take<int32_t>(J + 1); b.c_src = c.take<int32_t>(Cn);

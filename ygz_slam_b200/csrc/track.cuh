@@ -38,11 +38,7 @@ struct TrackBatch {
     // sparse alignment (SparseImgAlign::run): problem j owns scratch features [offsets[j], offsets[j] + n_feat[j])
     int32_t *ref_slot, *cur_slot, *offsets, *in_off, *n_feat, *n_meas;
     double *T_ref, *T_cur;      // [J][12]; T_cur: reference pose in, aligned pose, then pose-only result
-    float *ref_patch, *gdx, *gdy;
-    double* frame_jac;
-    uint8_t* visible;
-    double* sparse_ws;
-    void* sa2_scratch;          // global fall-back of the second-generation kernel's per-feature staging
+    void* feat_scratch;         // [J * cells] features: global fall-back of the kernel's per-feature staging
     // Matcher::SparseImageAlignment's motion check, poses relative to the local key-frames
     int32_t* aligned;           // [J]
     double* rel;                // [J][kTrackMaxLocal][12]
@@ -68,6 +64,5 @@ int launch_pose_only_dev(ygzb_ctx* ctx, int n_problems, const int32_t* d_offsets
                          const double* d_px, double* d_T_cw, uint8_t* d_inlier, double* d_depth, int32_t* d_n_inlier, uint8_t* d_enable,
                          double* d_ws, int cluster, int max_points);
 size_t pose_only_ws_doubles(int n_problems);
-size_t sparse_align2_scratch_bytes(int n_problems, int cells);
 
 }  // namespace ygzb
